@@ -82,6 +82,28 @@ def device_inputs(w, dev, seed, structure_seed=1234):
     return logits, targets, student, teacher, attn
 
 
+DUMP_BYTES = 60 << 20          # payload of all .npy files together; headers keep the total under 64 MB
+
+
+def dump_outputs(out_dir, arrays, budget=DUMP_BYTES):
+    """Writes {name: tensor} as out_dir/<name>.npy: float64 stays float64, every other dtype becomes float32 (exact for bf16).
+    Smaller arrays are written whole first; an array larger than its share of what is left of `budget` is written as the
+    1-D sample of its flattened elements at sorted flat indices drawn with numpy's default_rng(0), so runs with the same
+    arguments write the same elements."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    todo = sorted(arrays.items(), key=lambda kv: kv[1].numel())
+    left = budget
+    for i, (name, t) in enumerate(todo):
+        t = t.detach().cpu()
+        a = (t if t.dtype == torch.float64 else t.float()).numpy()
+        k = min(a.size, left // (len(todo) - i) // a.itemsize)
+        if k < a.size:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, k, replace=False))]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+        left -= a.nbytes
+
+
 # ------------------------------------------------------------------------------------------------ clocks
 class ClockSampler(threading.Thread):
     """One streaming `nvidia-smi -lms 50` process (a fresh nvidia-smi per sample takes longer than a short timed region)."""
@@ -267,7 +289,13 @@ def main():
     ap.add_argument("--views", action="store_true",
                     help="hand the tokens over as the CLS-stripped views out[:, 1:, :] of [B, N+1, D] tensors, like trainer.py:29 / teacher.py:157 do "
                          "(consumed in place; default: dense tensors)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what rank 0's last timed step returned (loss, gradients of the logits, of "
+                         "log_temperatures and of each student tensor) as DIR/<name>.npy, float32; arrays past a 60 MiB total "
+                         "are written as a fixed seeded sample of their elements (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference_arm(args)
         return
@@ -340,6 +368,10 @@ def main():
     clocks = sampler.finish()
     ms_total = e0.elapsed_time(e1)
     launches = int(lib.basd_launch_count())
+    if args.dump_outputs and rank == 0:
+        outs = {"loss": loss, "grad_logits": logits.grad, "grad_log_temperatures": m.layer_selector.log_temperatures.grad}
+        outs.update({f"grad_student_{l}": t.grad for l, t in student.items()})
+        dump_outputs(args.dump_outputs, outs)
     # per-kernel breakdown: the same steps again with a CUDA-event bracket around every launch group (kept out of the
     # timed region above: ~150 event records per step cost 0.1-0.2 ms and keep consecutive kernels from overlapping)
     lib.basd_timing_reset()

@@ -487,7 +487,7 @@ def test_two_rank_nccl_on_two_gpus_matches_single_process(lib, cuda_dev, tmp_pat
     mixing weights, temperature gradients and the concatenated student gradients of two ranks on two B200s against a
     single process on the whole batch.  Skipped on single-GPU boxes."""
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs two GPUs (gpurun --gpus 2)")
+        pytest.skip("needs two GPUs")
     _two_rank_case(cuda_dev, tmp_path, {})
 
 
