@@ -37,7 +37,7 @@ typedef struct basd_shape {
     int Lt;         /* teacher layers handed over (sorted keys, layer_selector.py:123) */
     int P;          /* student extraction points (combined.py:34-40)                  */
     int H;          /* attention heads (1 for CNN teachers, teacher.py:188-191)       */
-    int has_cls;    /* teacher_has_cls_token (combined.py:27)                         */
+    int has_cls;    /* teacher_has_cls_token (combined.py:27), or BASD_ATTN_QUERY_MEAN  */
     int act_dtype;  /* BASD_DTYPE_* of student and teacher tokens                     */
     int attn_dtype; /* BASD_DTYPE_* of attention maps                                 */
     int world_size; /* ranks whose pooled statistics are summed (equal local batches) */
@@ -56,6 +56,14 @@ typedef struct basd_shape {
  *                       phases 1-2 stop at view "w" [P*Lt] (attention pointers are not read, geo_loss = 0); phase 3 is a no-op;
  *                       phase 4 takes d(total)/d(w) from view "gw" (written by the caller, *grad_geo multiplies it) and returns
  *                       the gradients w.r.t. the student tensors and log_temperatures through the closed-form selector backward. */
+/* basd_shape.has_cls
+ *   0                     no CLS token: every attention pointer holds the full map [B,H,Nt,Nt] (relational.py:27 averages it
+ *                         over heads and queries).
+ *   1                     CLS token: the full map [B,H,Nt+1,Nt+1] or its CLS query row [B,H,1,Nt+1] (relational.py:24).
+ *   BASD_ATTN_QUERY_MEAN  no CLS token, and every attention pointer holds the query-mean row per head [B,H,1,Nt]
+ *                         (basd_query_mean_attention): what relational.py:27 reads of the full map, without the map. */
+#define BASD_ATTN_QUERY_MEAN 2
+
 #define BASD_MODE_LOSS 0
 #define BASD_MODE_PAIR 1
 #define BASD_MODE_SELECTOR 2
@@ -63,7 +71,7 @@ typedef struct basd_shape {
 typedef struct basd_inputs {
     const void* student[BASD_MAX_POINTS];   /* P  tensors [B,Ns,Ds]; element strides below            */
     const void* teacher[BASD_MAX_LAYERS];   /* Lt tensors [B,Nt,Dt]                                   */
-    const void* attn[BASD_MAX_LAYERS];      /* Lt tensors [B,H,Nt+1,Nt+1] (has_cls) or [B,H,Nt,Nt]    */
+    const void* attn[BASD_MAX_LAYERS];      /* Lt tensors [B,H,Nt+1,Nt+1] (has_cls) or [B,H,Nt,Nt]; rows: see has_cls */
     int64_t student_strides[3];             /* (batch, token, feature) in elements, same for all P    */
     int64_t teacher_strides[3];
     int64_t attn_strides[4];                /* (batch, head, query, key)                              */
@@ -113,6 +121,17 @@ int basd_mp_rank(const void* features, int64_t M, int D, int dtype, int64_t row_
  * by basd_forward_stats in place of the [B,H,S,S] map (attn_strides accordingly). */
 int basd_cls_attention_rows(const void* q, const void* k, int dtype, int B, int H, int S, int dh, const int64_t* q_strides,
                             const int64_t* k_strides, float scale, float* out, void* stream);
+
+/* The same for teachers WITHOUT a CLS token (relational.py:27 reads attn.mean over heads and all queries): emits the
+ * query mean of every head's map, out[b,h,:] = (1/S) sum_q softmax_s(q[b,h,q,:] . k[b,h,s,:] * scale), fp32 [B,H,S], and never
+ * stores an S x S map (two passes of tcgen05 products over q and k: row max / sum of exps per query, then the normalised
+ * probabilities summed per key; fixed-order sums, bitwise repeatable).  q, k: [B,H,S,dh] with element strides (b,h,s,d),
+ * d stride 1 (views into a fused qkv tensor are fine); dtype BASD_DTYPE_BF16, or BASD_DTYPE_F32 (split-bf16 products,
+ * fp32-class accuracy).  dh a multiple of 8 up to 256, 1 <= S <= 2048; base 16-byte aligned, (b,h,s) strides multiples of 8
+ * (bf16) or 4 (fp32) elements.  The result, viewed as [B,H,1,S], is accepted by basd_forward_stats with
+ * has_cls = BASD_ATTN_QUERY_MEAN in place of the [B,H,S,S] map. */
+int basd_query_mean_attention(const void* q, const void* k, int dtype, int B, int H, int S, int dh, const int64_t* q_strides,
+                              const int64_t* k_strides, float scale, float* out, void* stream);
 
 /* Host-resident teacher attention (an offline / CPU-resident teacher): copies the CLS query rows of a HOST map [B,H,S,S]
  * (element strides (b,h,q,k), k stride 1, 2- or 4-byte elements) to a dense DEVICE tensor [B,H,1,S] with one pitched DMA -

@@ -9,6 +9,7 @@ MAX_POINTS = 8
 MAX_LAYERS = 64
 DTYPE_F32, DTYPE_BF16 = 0, 1
 MODE_LOSS, MODE_PAIR, MODE_SELECTOR = 0, 1, 2
+ATTN_QUERY_MEAN = 2             # basd_shape.has_cls: no CLS token, attention given as query-mean rows [B,H,1,Nt]
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("BASD_B200_LIB") or os.path.join(_HERE, "libbasd_b200.so")      # (override: A/B runs of two builds)
@@ -39,7 +40,7 @@ EXPORTS = [
     "basd_last_error", "basd_version", "basd_timing_enable", "basd_timing_reset", "basd_launch_count", "basd_timing_slots",
     "basd_timing_name", "basd_timing_read", "basd_polar_steps", "basd_polar_launches_per_step", "basd_cls_attention_rows",
     "basd_copy_cls_rows_h2d", "basd_debug_polar_clocks", "basd_debug_spectral_clocks", "basd_align_tokens", "basd_align_tokens_bwd",
-    "basd_uwso_combine",
+    "basd_uwso_combine", "basd_query_mean_attention",
 ]
 
 _lib = None
@@ -73,6 +74,8 @@ def load():
     lib.basd_selftest_eig.argtypes = [vp, ctypes.c_int, vp, vp, vp, vp, vp]
     lib.basd_cls_attention_rows.argtypes = [vp, vp, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int,
                                             ctypes.POINTER(ctypes.c_int64), ctypes.POINTER(ctypes.c_int64), ctypes.c_float, vp, vp]
+    lib.basd_query_mean_attention.argtypes = [vp, vp, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int,
+                                              ctypes.POINTER(ctypes.c_int64), ctypes.POINTER(ctypes.c_int64), ctypes.c_float, vp, vp]
     lib.basd_copy_cls_rows_h2d.argtypes = [vp, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.POINTER(ctypes.c_int64), vp, vp]
     lib.basd_align_tokens.argtypes = [vp, ctypes.c_int, ctypes.POINTER(ctypes.c_int64), ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, vp, vp]
     lib.basd_align_tokens_bwd.argtypes = [vp, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, vp, vp]

@@ -213,6 +213,7 @@ Layout make_layout(const basd_shape& s) {
 int check_shape(const basd_shape& s) {
     if (s.B < 1 || s.Ns < 2 || s.Nt < 1 || s.Lt < 1 || s.P < 1) return fail("invalid shape");
     if (s.world_size < 1) return fail("world_size must be >= 1");
+    if (s.has_cls < 0 || s.has_cls > BASD_ATTN_QUERY_MEAN) return fail("basd_shape.has_cls must be 0, 1 or BASD_ATTN_QUERY_MEAN (2), got %d", s.has_cls);
     if (s.mode < BASD_MODE_LOSS || s.mode > BASD_MODE_SELECTOR) return fail("unknown basd_shape.mode %d", s.mode);
     if (s.mode == BASD_MODE_PAIR && (s.Lt != 1 || s.P != 1)) return fail("BASD_MODE_PAIR takes one student and one teacher tensor (Lt = P = 1)");
     if (s.P > BASD_MAX_POINTS || s.Lt > BASD_MAX_LAYERS) return fail("P <= %d and Lt <= %d required", BASD_MAX_POINTS, BASD_MAX_LAYERS);
@@ -616,6 +617,37 @@ extern "C" int basd_cls_attention_rows(const void* q, const void* k, int dtype, 
     const long long qs[2] = {q_strides[0], q_strides[1]};
     const long long ks[3] = {k_strides[0], k_strides[1], k_strides[2]};
     CK(launch_cls_attention_rows(q, k, dtype == BASD_DTYPE_BF16, B, H, S, dh, qs, ks, scale, out, reinterpret_cast<cudaStream_t>(stream)));
+    return 0;
+}
+
+// ------------------------------------------------------------------------------------------- query-mean attention rows
+extern "C" int basd_query_mean_attention(const void* q, const void* k, int dtype, int B, int H, int S, int dh, const int64_t* q_strides,
+                                         const int64_t* k_strides, float scale, float* out, void* stream) {
+    if (!q || !k || !out || !q_strides || !k_strides) return fail("null argument");
+    if (dtype != BASD_DTYPE_F32 && dtype != BASD_DTYPE_BF16) return fail("basd_query_mean_attention: unknown dtype %d", dtype);
+    if (B < 1 || H < 1 || static_cast<long long>(B) * H > 0x7fffffffLL) return fail("basd_query_mean_attention: invalid B=%d, H=%d", B, H);
+    if (S < 1 || S > kQueryMeanMaxTokens) return fail("basd_query_mean_attention: S=%d outside 1..%d", S, kQueryMeanMaxTokens);
+    if (dh < 8 || dh > kQueryMeanMaxHeadDim || dh % 8)
+        return fail("basd_query_mean_attention: dh=%d must be a multiple of 8 in 8..%d", dh, kQueryMeanMaxHeadDim);
+    if (q_strides[3] != 1 || k_strides[3] != 1) return fail("basd_query_mean_attention: the head-dim stride of q and k must be 1");
+    // The stride of a size-1 dimension is arbitrary (frameworks report anything there): replace it by the packed one.
+    long long qs[3], ks[3];
+    const int64_t* in[2] = {q_strides, k_strides};
+    long long* o[2] = {qs, ks};
+    for (int i = 0; i < 2; ++i) {
+        o[i][2] = S == 1 ? dh : in[i][2];
+        o[i][1] = H == 1 ? static_cast<long long>(S) * o[i][2] : in[i][1];
+        o[i][0] = B == 1 ? static_cast<long long>(H) * o[i][1] : in[i][0];
+    }
+    // bf16 operands are read by TMA (16-byte aligned base and strides); fp32 rows as 16-byte vectors
+    const long long align = dtype == BASD_DTYPE_BF16 ? 8 : 4;
+    for (int i = 0; i < 2; ++i) {
+        const void* p = i ? k : q;
+        if ((reinterpret_cast<uintptr_t>(p) & 15) || o[i][0] < 1 || o[i][1] < 1 || o[i][2] < 1 || o[i][0] % align || o[i][1] % align || o[i][2] % align)
+            return fail("basd_query_mean_attention: %s needs a 16-byte aligned base and positive (b,h,s) strides that are multiples of %lld elements "
+                        "(got %p, %lld,%lld,%lld)", i ? "k" : "q", align, p, o[i][0], o[i][1], o[i][2]);
+    }
+    CK(launch_query_mean_attention(q, k, dtype == BASD_DTYPE_BF16, B, H, S, dh, qs, ks, scale, out, reinterpret_cast<cudaStream_t>(stream)));
     return 0;
 }
 

@@ -60,6 +60,24 @@ static int make_map(CUtensorMap* map, const void* ptr, uint64_t inner, uint64_t 
     return 0;
 }
 
+// bf16 tensor of any rank with explicit byte strides (dims[0] contiguous); box[0] = 64 (128-byte rows); SWIZZLE_128B; OOB -> zeros.
+// For the other translation units (attention_rows.cu: 4-D maps over strided q / k views).
+int tensor_map_encode_bf16(CUtensorMap* map, int rank, const void* ptr, const uint64_t* dims, const uint64_t* strides_bytes, const uint32_t* box) {
+    if (gemm_init_driver_api()) return 1;
+    cuuint64_t d[5], s[4];
+    cuuint32_t bx[5], estr[5];
+    for (int i = 0; i < rank; ++i) { d[i] = dims[i]; bx[i] = box[i]; estr[i] = 1; }
+    for (int i = 0; i + 1 < rank; ++i) s[i] = strides_bytes[i];
+    CUresult r = g_encode(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, rank, const_cast<void*>(ptr), d, s, bx, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                          CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    if (r != CUDA_SUCCESS) {
+        snprintf(g_gemm_err, sizeof g_gemm_err, "cuTensorMapEncodeTiled (rank %d) failed (%d) ptr=%p dims=%llu,%llu strides=%llu,%llu", rank, (int)r, ptr,
+                 (unsigned long long)dims[0], (unsigned long long)dims[1], (unsigned long long)strides_bytes[0], (unsigned long long)strides_bytes[1]);
+        return 1;
+    }
+    return 0;
+}
+
 // fp32 tensor viewed as [batch][rows][inner]; box = [1][32][32] (128-byte rows); SWIZZLE_128B; OOB -> zeros.
 static int make_map_f32(CUtensorMap* map, const void* ptr, uint64_t inner, uint64_t rows, uint64_t batch, uint64_t row_pitch_elems,
                         uint64_t batch_pitch_elems) {

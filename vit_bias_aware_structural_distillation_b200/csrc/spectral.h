@@ -74,6 +74,12 @@ size_t wgrad_part_floats(int P, int Lt);
 cudaError_t launch_cls_attention_rows(const void* q, const void* k, int is_bf16, int B, int H, int S, int dh,
                                       const long long* q_strides /*[b,h]*/, const long long* k_strides /*[b,h,s]*/, float scale,
                                       float* out /*[B,H,S]*/, cudaStream_t st);
+// (attention_rows.cu) out[b,h,s] = mean over queries of softmax(scale q k^T)[., s], fp32 [B,H,S]; q, k [B,H,S,dh] with (b,h,s)
+// element strides, d stride 1.  bf16: 16-byte aligned base and strides; fp32: 16-byte aligned base, strides multiples of 4.
+constexpr int kQueryMeanMaxTokens = 2048, kQueryMeanMaxHeadDim = 256;
+cudaError_t launch_query_mean_attention(const void* q, const void* k, int is_bf16, int B, int H, int S, int dh,
+                                        const long long* q_strides /*[b,h,s]*/, const long long* k_strides /*[b,h,s]*/, float scale,
+                                        float* out /*[B,H,S]*/, cudaStream_t st);
 // standalone combined.py:9-14 (tokens [B,Nin,D] with element strides -> dense [B,Nout,D]) and its adjoint (dense in, dense out)
 cudaError_t launch_align_tokens(const void* src, int is_bf16, long long sb, long long sn, long long sd, int B, int Nin, int Nout, int D,
                                 void* dst, cudaStream_t st);

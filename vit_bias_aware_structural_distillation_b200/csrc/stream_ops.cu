@@ -42,7 +42,13 @@ __global__ void importance_rows_kernel(PtrTable attn, int B, int H, int Nt, int 
     const int b = blockIdx.x, j = blockIdx.y;
     const T* A = reinterpret_cast<const T*>(attn.p[j]) + static_cast<long long>(b) * sb;
     float* out = rows + (static_cast<size_t>(j) * B + b) * Nt;
-    if (has_cls) {
+    if (has_cls == 2) {                                 // BASD_ATTN_QUERY_MEAN: [B,H,1,Nt] rows already averaged over the queries
+        for (int n = threadIdx.x; n < Nt; n += blockDim.x) {
+            float s = 0.f;
+            for (int h = 0; h < H; ++h) s += ld_as_float(A + h * sh + n * sk);
+            out[n] = s / static_cast<float>(H);
+        }
+    } else if (has_cls) {
         for (int n = threadIdx.x; n < Nt; n += blockDim.x) {
             float s = 0.f;
             for (int h = 0; h < H; ++h) s += ld_as_float(A + h * sh + (1 + n) * sk);     // query 0 (CLS), keys 1..Nt

@@ -26,7 +26,7 @@ import torch.nn as nn
 import torch.nn.functional as F
 
 from . import _lib
-from ._lib import DTYPE_BF16, DTYPE_F32, MODE_LOSS, MODE_PAIR, MODE_SELECTOR, Inputs, Shape
+from ._lib import ATTN_QUERY_MEAN, DTYPE_BF16, DTYPE_F32, MODE_LOSS, MODE_PAIR, MODE_SELECTOR, Inputs, Shape
 
 
 # --------------------------------------------------------------------------------------------- low-level plumbing
@@ -102,15 +102,21 @@ def _prepare(students: Sequence[torch.Tensor], teachers: Sequence[torch.Tensor],
         if log_temperatures.numel() != len(students):
             raise _lib.BasdError(f"{log_temperatures.numel()} log_temperatures for {len(students)} student extraction points")
     H = attns[0].shape[1] if attns else 1
+    attn_code = int(has_cls)
     if attns:
         exp_attn = (B, H, Nt + 1, Nt + 1) if has_cls else (B, H, Nt, Nt)
-        cls_rows_only = (B, H, 1, Nt + 1)          # HostStager hands over just the CLS query row (all relational.py:24 reads)
-        if tuple(attns[0].shape) != exp_attn and not (has_cls and tuple(attns[0].shape) == cls_rows_only):
-            raise _lib.BasdError(f"attention shape {tuple(attns[0].shape)} != expected {exp_attn}")
+        # rows only: the CLS query row (HostStager, cls_attention_rows; all relational.py:24 reads) or, without a CLS token, the
+        # query mean per head (query_mean_attention; all relational.py:27 reads)
+        rows_only = (B, H, 1, Nt + 1) if has_cls else (B, H, 1, Nt)
+        got = tuple(attns[0].shape)
+        if got not in (exp_attn, rows_only):
+            raise _lib.BasdError(f"attention shape {got} != expected {exp_attn} (or rows {rows_only})")
+        if not has_cls and got != exp_attn:
+            attn_code = ATTN_QUERY_MEAN
     proj_s = proj_s.detach().to(device=dev, dtype=torch.float32).contiguous()
     proj_t = proj_t.detach().to(device=dev, dtype=torch.float32).contiguous()
     logt = log_temperatures.detach().to(device=dev, dtype=torch.float32).contiguous()
-    shape = Shape(B=B, Ns=Ns, Nt=Nt, Ds=Ds, Dt=Dt, Lt=len(teachers), P=len(students), H=H, has_cls=int(has_cls),
+    shape = Shape(B=B, Ns=Ns, Nt=Nt, Ds=Ds, Dt=Dt, Lt=len(teachers), P=len(students), H=H, has_cls=attn_code,
                   act_dtype=_dtype_code(students[0]), attn_dtype=_dtype_code(attns[0]) if attns else DTYPE_F32, world_size=world_size,
                   polar_steps=int(polar_steps), mode=int(mode))
     inp = Inputs()
@@ -288,7 +294,8 @@ class HostStager:
     offline / CPU-resident teacher): double-buffered device slots, copies issued on a dedicated copy stream so that the
     transfer of step i+1 overlaps the loss of step i.  Of every teacher attention map `[B,H,N+1,N+1]` only the CLS query
     row is gathered and copied (relational.py:24 reads nothing else): 14.5 MB instead of 2.9 GB per step at
-    BASELINE.json configs[1].  CNN teachers (no CLS, relational.py:27) need the whole map and get it.
+    BASELINE.json configs[1].  Teachers without a CLS token (relational.py:27) get whatever they hand over copied as it is:
+    the whole map [B,H,N,N], or - from `query_mean_attention` - the query-mean rows [B,H,1,N], 1/N of the map's bytes.
 
         stager = HostStager(loss_module)
         h = stager.submit(logits, targets, student, teacher_tokens, teacher_attns)   # host tensors (pinned = async)
@@ -407,6 +414,41 @@ def cls_attention_rows(q: torch.Tensor, k: torch.Tensor, scale: float | None = N
         ks = (ctypes.c_int64 * 4)(*k.stride())
         _lib.check(lib.basd_cls_attention_rows(q.data_ptr(), k.data_ptr(), _dtype_code(q), B, H, S, dh, qs, ks, float(scale), out.data_ptr(),
                                                _stream_ptr(q.device)), "basd_cls_attention_rows")
+    return out
+
+
+def query_mean_attention(q: torch.Tensor, k: torch.Tensor, scale: float | None = None) -> torch.Tensor:
+    """Query mean of every head's softmax(q k^T * scale), shape [B, H, 1, S] fp32, straight from q and k [B, H, S, dh] (strided
+    views of a fused qkv tensor are fine; dh a multiple of 8 up to 256, S up to 2048).  For teachers WITHOUT a CLS token
+    relational.py:27 reads the attention only as attn.mean over heads and queries: pass the result as `all_teacher_attns[j]`
+    (with teacher_has_cls_token=False) instead of the full [B, H, S, S] map the reference hook (src/models/teacher.py:27-39)
+    materialises.  The kernel never stores an S x S map; fp32 inputs run as split-bf16 products (fp32-class accuracy)."""
+    if q.dim() != 4 or tuple(k.shape) != tuple(q.shape):
+        raise _lib.BasdError(f"query_mean_attention: q {tuple(q.shape)} and k {tuple(k.shape)} must both be [B, H, S, dh]")
+    lib = _lib.load()
+    if q.device.type != "cuda" or k.device.type != "cuda":
+        raise _lib.BasdError("query_mean_attention: CUDA tensors required (no CPU fallback)")
+    if k.device != q.device:
+        raise _lib.BasdError(f"query_mean_attention: q on {q.device} and k on {k.device}")
+    if q.dtype != k.dtype or q.dtype not in (torch.float32, torch.bfloat16):
+        q, k = q.float(), k.float()
+    B, H, S, dh = q.shape
+
+    def aligned(t):             # read in place: d stride 1, 16-byte aligned base and (b, h, s) strides
+        e = 8 if t.dtype == torch.bfloat16 else 4
+        return t.stride(3) == 1 and t.data_ptr() % 16 == 0 and all(t.stride(i) % e == 0 or t.shape[i] == 1 for i in range(3))
+    if not aligned(q):
+        q = q.contiguous()
+    if not aligned(k):
+        k = k.contiguous()
+    if scale is None:
+        scale = dh ** -0.5
+    with torch.cuda.device(q.device):
+        out = torch.empty(B, H, 1, S, dtype=torch.float32, device=q.device)
+        qs = (ctypes.c_int64 * 4)(*q.stride())
+        ks = (ctypes.c_int64 * 4)(*k.stride())
+        _lib.check(lib.basd_query_mean_attention(q.data_ptr(), k.data_ptr(), _dtype_code(q), B, H, S, dh, qs, ks, float(scale), out.data_ptr(),
+                                                 _stream_ptr(q.device)), "basd_query_mean_attention")
     return out
 
 
