@@ -27,6 +27,9 @@ extern "C" {
 
 #define BASD_DTYPE_F32 0
 #define BASD_DTYPE_BF16 1
+/* basd_shape.act_dtype only: fp32 tokens carried as split-bf16 pairs hi = bf16(x), lo = bf16(x - hi) instead of being rounded
+ * to bf16 on entry (every product reads them as hi*hi + hi*lo + lo*hi, every streaming kernel as hi + lo; fp32-class accuracy) */
+#define BASD_DTYPE_F32_SPLIT 2
 #define BASD_MAX_POINTS 8
 #define BASD_MAX_LAYERS 64
 
@@ -38,8 +41,9 @@ typedef struct basd_shape {
     int P;          /* student extraction points (combined.py:34-40)                  */
     int H;          /* attention heads (1 for CNN teachers, teacher.py:188-191)       */
     int has_cls;    /* teacher_has_cls_token (combined.py:27), or BASD_ATTN_QUERY_MEAN  */
-    int act_dtype;  /* BASD_DTYPE_* of student and teacher tokens                     */
-    int attn_dtype; /* BASD_DTYPE_* of attention maps                                 */
+    int act_dtype;  /* BASD_DTYPE_* of student and teacher tokens: BASD_DTYPE_BF16 (read in place), BASD_DTYPE_F32 (rounded
+                       to bf16 on entry) or BASD_DTYPE_F32_SPLIT (fp32 tokens kept as split-bf16 pairs; more workspace) */
+    int attn_dtype; /* BASD_DTYPE_F32 or BASD_DTYPE_BF16 of attention maps                                          */
     int world_size; /* ranks whose pooled statistics are summed (equal local batches) */
     int polar_steps;/* Newton-Schulz steps of the Procrustes polar iteration: 0 = default (10: singular values of the
                        cross-covariance down to 3e-5 ||C||_F), up to 16 (each step more divides that floor by ~4);

@@ -8,6 +8,7 @@ import os
 MAX_POINTS = 8
 MAX_LAYERS = 64
 DTYPE_F32, DTYPE_BF16 = 0, 1
+DTYPE_F32_SPLIT = 2             # basd_shape.act_dtype: fp32 tokens carried as split-bf16 pairs (token_precision="fp32")
 MODE_LOSS, MODE_PAIR, MODE_SELECTOR = 0, 1, 2
 ATTN_QUERY_MEAN = 2             # basd_shape.has_cls: no CLS token, attention given as query-mean rows [B,H,1,Nt]
 

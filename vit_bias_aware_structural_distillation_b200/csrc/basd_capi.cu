@@ -129,9 +129,10 @@ Layout make_layout(const basd_shape& s) {
     L.rows = take(4 * Lt * B * Nt);
     L.pt_hi = take(2 * Ds * Dt);
     L.pt_lo = take(2 * Ds * Dt);
-    const bool pack = s.act_dtype == BASD_DTYPE_F32;
-    L.tpk = take(pack ? 2 * Lt * B * Nt * Dt : 0);
-    L.spk = take(pack ? 2 * P * B * Ns * Ds : 0);
+    // fp32 tokens are packed to dense bf16 [layer or point][B][N][D]; split-bf16 pairs as a hi block then a lo block
+    const size_t pack = s.act_dtype == BASD_DTYPE_F32 ? 1 : s.act_dtype == BASD_DTYPE_F32_SPLIT ? 2 : 0;
+    L.tpk = take(pack * 2 * Lt * B * Nt * Dt);
+    L.spk = take(pack * 2 * P * B * Ns * Ds);
     L.z = take(2 * 2 * Lt * B * (Nt + 1) * Ds);    // projected teacher tokens, split pair: hi block then lo block (rows of a CLS-stripped view: B (Nt + 1) - 1)
     L.stats = take(4 * (Lt + P) * (Ds * Ds + Ds));
     L.ranks = take(4 * Lt);
@@ -213,6 +214,10 @@ Layout make_layout(const basd_shape& s) {
 int check_shape(const basd_shape& s) {
     if (s.B < 1 || s.Ns < 2 || s.Nt < 1 || s.Lt < 1 || s.P < 1) return fail("invalid shape");
     if (s.world_size < 1) return fail("world_size must be >= 1");
+    if (s.act_dtype < BASD_DTYPE_F32 || s.act_dtype > BASD_DTYPE_F32_SPLIT)
+        return fail("basd_shape.act_dtype must be BASD_DTYPE_F32 (0), BASD_DTYPE_BF16 (1) or BASD_DTYPE_F32_SPLIT (2), got %d", s.act_dtype);
+    if (s.attn_dtype != BASD_DTYPE_F32 && s.attn_dtype != BASD_DTYPE_BF16)
+        return fail("basd_shape.attn_dtype must be BASD_DTYPE_F32 (0) or BASD_DTYPE_BF16 (1), got %d", s.attn_dtype);
     if (s.has_cls < 0 || s.has_cls > BASD_ATTN_QUERY_MEAN) return fail("basd_shape.has_cls must be 0, 1 or BASD_ATTN_QUERY_MEAN (2), got %d", s.has_cls);
     if (s.mode < BASD_MODE_LOSS || s.mode > BASD_MODE_SELECTOR) return fail("unknown basd_shape.mode %d", s.mode);
     if (s.mode == BASD_MODE_PAIR && (s.Lt != 1 || s.P != 1)) return fail("BASD_MODE_PAIR takes one student and one teacher tensor (Lt = P = 1)");
@@ -238,13 +243,20 @@ bool cls_view3(const int64_t* st, int N, int D) { return st[2] == 1 && st[1] == 
 struct Resolved {
     const __nv_bfloat16* teacher[BASD_MAX_LAYERS];
     const __nv_bfloat16* student[BASD_MAX_POINTS];
+    const __nv_bfloat16* teacher_lo[BASD_MAX_LAYERS];     // split-bf16 tokens (BASD_DTYPE_F32_SPLIT): lo halves; null otherwise
+    const __nv_bfloat16* student_lo[BASD_MAX_POINTS];
     long long teacher_bs, student_bs;       // batch strides in elements
     int teacher_gap, student_gap;           // 1: rows of the tensor read as a flat matrix carry one foreign row between samples
 };
 
-// After phase 1 the bf16, dense versions of the tokens are either the inputs themselves or the packed copies.
+// After phase 1 the bf16, dense versions of the tokens are either the inputs themselves or the packed copies (hi and lo
+// halves of split pairs).
+bool packs(const basd_shape& s) { return s.act_dtype == BASD_DTYPE_F32 || s.act_dtype == BASD_DTYPE_F32_SPLIT; }
 int resolve(const basd_shape& s, const basd_inputs& in, uint8_t* ws, const Layout& L, Resolved* r) {
-    const bool pack = s.act_dtype == BASD_DTYPE_F32;
+    const bool pack = packs(s), split = s.act_dtype == BASD_DTYPE_F32_SPLIT;
+    const size_t t_block = static_cast<size_t>(s.Lt) * s.B * s.Nt * s.Dt, s_block = static_cast<size_t>(s.P) * s.B * s.Ns * s.Ds;
+    memset(r->teacher_lo, 0, sizeof r->teacher_lo);
+    memset(r->student_lo, 0, sizeof r->student_lo);
     r->teacher_bs = static_cast<long long>(s.Nt) * s.Dt; r->student_bs = static_cast<long long>(s.Ns) * s.Ds;
     r->teacher_gap = 0; r->student_gap = 0;
     if (!pack) {
@@ -263,12 +275,14 @@ int resolve(const basd_shape& s, const basd_inputs& in, uint8_t* ws, const Layou
         r->teacher[j] = pack ? reinterpret_cast<const __nv_bfloat16*>(ws + L.tpk) + static_cast<size_t>(j) * s.B * s.Nt * s.Dt
                              : reinterpret_cast<const __nv_bfloat16*>(in.teacher[j]);
         if (reinterpret_cast<uintptr_t>(r->teacher[j]) & 15) return fail("teacher tensor %d not 16-byte aligned", j);
+        if (split) r->teacher_lo[j] = r->teacher[j] + t_block;
     }
     for (int i = 0; i < s.P; ++i) {
         if (!in.student[i]) return fail("null student pointer at point %d", i);
         r->student[i] = pack ? reinterpret_cast<const __nv_bfloat16*>(ws + L.spk) + static_cast<size_t>(i) * s.B * s.Ns * s.Ds
                              : reinterpret_cast<const __nv_bfloat16*>(in.student[i]);
         if (reinterpret_cast<uintptr_t>(r->student[i]) & 15) return fail("student tensor %d not 16-byte aligned", i);
+        if (split) r->student_lo[i] = r->student[i] + s_block;
     }
     return 0;
 }
@@ -329,16 +343,21 @@ extern "C" int basd_forward_stats(const basd_shape* shape, const basd_inputs* in
     }
     __nv_bfloat16* pt_hi = reinterpret_cast<__nv_bfloat16*>(ws + L.pt_hi);
     __nv_bfloat16* pt_lo = reinterpret_cast<__nv_bfloat16*>(ws + L.pt_lo);
-    Scope* pack_scope = new Scope(1, st, 1 + (s.act_dtype == BASD_DTYPE_F32 ? s.Lt + s.P : 0));
+    Scope* pack_scope = new Scope(1, st, 1 + (packs(s) ? s.Lt + s.P : 0));
     struct ScopeDel { Scope* p; ~ScopeDel() { delete p; } } pack_del{pack_scope};
     if (selector) CK(launch_split_bf16(in.proj_t, pt_hi, pt_lo, static_cast<size_t>(s.Ds) * s.Dt, st));
-    if (s.act_dtype == BASD_DTYPE_F32) {
+    if (packs(s)) {
+        // fp32 tokens: rounded to bf16, or (BASD_DTYPE_F32_SPLIT) kept as split pairs, lo halves one block behind the hi halves
+        const bool split = s.act_dtype == BASD_DTYPE_F32_SPLIT;
+        __nv_bfloat16* tpk = reinterpret_cast<__nv_bfloat16*>(ws + L.tpk);
+        __nv_bfloat16* spk = reinterpret_cast<__nv_bfloat16*>(ws + L.spk);
+        const size_t t_block = static_cast<size_t>(s.Lt) * Mt * s.Dt, s_block = static_cast<size_t>(s.P) * Ms * s.Ds;
         for (int j = 0; j < s.Lt; ++j)
             CK(launch_pack_bf16(in.teacher[j], 0, in.teacher_strides[0], in.teacher_strides[1], in.teacher_strides[2], s.B, s.Nt, s.Dt,
-                                reinterpret_cast<__nv_bfloat16*>(ws + L.tpk) + static_cast<size_t>(j) * Mt * s.Dt, nullptr, st));
+                                tpk + static_cast<size_t>(j) * Mt * s.Dt, split ? tpk + t_block + static_cast<size_t>(j) * Mt * s.Dt : nullptr, st));
         for (int i = 0; i < s.P; ++i)
             CK(launch_pack_bf16(in.student[i], 0, in.student_strides[0], in.student_strides[1], in.student_strides[2], s.B, s.Ns, s.Ds,
-                                reinterpret_cast<__nv_bfloat16*>(ws + L.spk) + static_cast<size_t>(i) * Ms * s.Ds, nullptr, st));
+                                spk + static_cast<size_t>(i) * Ms * s.Ds, split ? spk + s_block + static_cast<size_t>(i) * Ms * s.Ds : nullptr, st));
     }
     delete pack_scope; pack_del.p = nullptr;
     Resolved r;
@@ -354,7 +373,7 @@ extern "C" int basd_forward_stats(const basd_shape* shape, const basd_inputs* in
         Scope sc(2, st, (s.Lt + 15) / 16);
         const void* layers[kMaxLayers];
         for (int j = 0; j < s.Lt; ++j) layers[j] = r.teacher[j];
-        CK(gemm_project(layers, s.Lt, Mt_rows, s.Dt, pt_hi, pt_lo, s.Ds, z, zlo, r.teacher_gap ? s.Nt + 1 : 0, s.Nt, st));
+        CK(gemm_project(layers, s.Lt, Mt_rows, s.Dt, pt_hi, pt_lo, s.Ds, z, zlo, r.teacher_gap ? s.Nt + 1 : 0, s.Nt, st, r.teacher_lo[0]));
     }
     {
         // Grams AND column sums in one pass over the operands (the ones-operand MMA of umma_gemm.cuh): Ds % 4 == 0 is implied by Ds % 8
@@ -363,10 +382,15 @@ extern "C" int basd_forward_stats(const basd_shape* shape, const basd_inputs* in
         float* gram_part = reinterpret_cast<float*>(ws + L.gram_part);
         const bool fused = gemm_gram_colsum_fused(s.Ds, true);
         CK(gemm_gram_batched(z, zlo, Mt_rows, s.Ds, s.Lt, stats, static_cast<long long>(stat_stride), gram_part, st, fused));
-        const void* pts[kMaxPoints];
-        for (int i = 0; i < s.P; ++i) pts[i] = r.student[i];
-        CK(gemm_gram_table(pts, s.P, Ms, s.Ds, stats + s.Lt * stat_stride, static_cast<long long>(stat_stride), gram_part,
-                           r.student_gap ? s.Ns : 0, r.student_bs, st, fused));
+        if (r.student_lo[0]) {                  // split-bf16 students (packed: one [P][Ms][Ds] block per half): three-term Grams
+            CK(gemm_gram_batched(r.student[0], r.student_lo[0], Ms, s.Ds, s.P, stats + s.Lt * stat_stride, static_cast<long long>(stat_stride),
+                                 gram_part, st, fused));
+        } else {
+            const void* pts[kMaxPoints];
+            for (int i = 0; i < s.P; ++i) pts[i] = r.student[i];
+            CK(gemm_gram_table(pts, s.P, Ms, s.Ds, stats + s.Lt * stat_stride, static_cast<long long>(stat_stride), gram_part,
+                               r.student_gap ? s.Ns : 0, r.student_bs, st, fused));
+        }
         delete sc; sc = nullptr;
         if (!fused) {                           // D_s > 192 (two-tile Grams): separate column-sum kernels
             const bool one_launch = Mt_rows == Ms && !r.student_gap;
@@ -378,11 +402,11 @@ extern "C" int basd_forward_stats(const basd_shape* shape, const basd_inputs* in
                 jt.out[j] = stats + j * stat_stride + static_cast<size_t>(s.Ds) * s.Ds;
             }
             for (int i = 0; i < s.P; ++i) {
-                js.hi[i] = r.student[i]; js.lo[i] = nullptr;
+                js.hi[i] = r.student[i]; js.lo[i] = r.student_lo[i];
                 js.out[i] = stats + (s.Lt + i) * stat_stride + static_cast<size_t>(s.Ds) * s.Ds;
             }
             if (one_launch) {                   // same row count, same addressing: one launch covers teacher and student jobs
-                for (int i = 0; i < s.P; ++i) { jt.hi[s.Lt + i] = js.hi[i]; jt.lo[s.Lt + i] = nullptr; jt.out[s.Lt + i] = js.out[i]; }
+                for (int i = 0; i < s.P; ++i) { jt.hi[s.Lt + i] = js.hi[i]; jt.lo[s.Lt + i] = js.lo[i]; jt.out[s.Lt + i] = js.out[i]; }
                 CK(launch_colsum(jt, s.Lt + s.P, Mt_rows, s.Ds, reinterpret_cast<float*>(ws + L.colsum_part), st));
             } else {
                 CK(launch_colsum(jt, s.Lt, Mt_rows, s.Ds, reinterpret_cast<float*>(ws + L.colsum_part), st));
@@ -439,14 +463,17 @@ extern "C" int basd_forward_solve(const basd_shape* shape, const basd_inputs* in
     __nv_bfloat16* tlo = reinterpret_cast<__nv_bfloat16*>(ws + L.tbar_lo);
     // teacher-token form: the mixed teacher stays on its own token grid (the resampling is folded into F, polar.cu)
     const bool vt = L.path == kPathTeacherTokens;
-    TIMED(8, 1, CK(launch_mix_teacher(tt, w, s.Lt, s.P, s.B, s.Nt, L.Nk, s.Dt, thi, tlo, st, r.teacher_bs)));
+    PtrTable tt_lo;
+    memset(&tt_lo, 0, sizeof tt_lo);
+    for (int j = 0; j < s.Lt; ++j) tt_lo.p[j] = r.teacher_lo[j];
+    TIMED(8, 1, CK(launch_mix_teacher(tt, w, s.Lt, s.P, s.B, s.Nt, L.Nk, s.Dt, thi, tlo, st, r.teacher_bs, r.teacher_lo[0] ? &tt_lo : nullptr)));
     float* ktt = reinterpret_cast<float*>(ws + L.ktt);
     TIMED(9, 1, CK(gemm_token_gram(thi, tlo, s.P * s.B, L.Nk, s.Dt, ktt, st)));
 
     PolarArgs pa;
     memset(&pa, 0, sizeof pa);
     pa.Ns = s.Ns; pa.Ds = s.Ds; pa.B = s.B; pa.P = s.P; pa.NsPad = L.NsPad; pa.n_problems = s.P * s.B;
-    for (int i = 0; i < s.P; ++i) pa.student[i] = r.student[i];
+    for (int i = 0; i < s.P; ++i) { pa.student[i] = r.student[i]; pa.student_lo[i] = r.student_lo[i]; }
     pa.student_bs = r.student_bs;
     pa.Ktt = ktt; pa.a = a; pa.ssum = ssum;
     {
@@ -515,9 +542,10 @@ extern "C" int basd_backward_dots(const basd_shape* shape, const basd_inputs* in
     if (s.mode != BASD_MODE_LOSS) return 0;      // PAIR: no mixing weights to differentiate; SELECTOR: d total / d w comes from the caller
     Resolved r;
     if (resolve(s, *in_, ws, L, &r)) return 1;
-    PtrTable tt;
+    PtrTable tt, tt_lo;
     memset(&tt, 0, sizeof tt);
-    for (int j = 0; j < s.Lt; ++j) tt.p[j] = r.teacher[j];
+    memset(&tt_lo, 0, sizeof tt_lo);
+    for (int j = 0; j < s.Lt; ++j) { tt.p[j] = r.teacher[j]; tt_lo.p[j] = r.teacher_lo[j]; }
     __nv_bfloat16* thi = reinterpret_cast<__nv_bfloat16*>(ws + L.tbar_hi);
     __nv_bfloat16* tlo = reinterpret_cast<__nv_bfloat16*>(ws + L.tbar_lo);
     __nv_bfloat16* dtm = reinterpret_cast<__nv_bfloat16*>(ws + L.dtm);
@@ -527,7 +555,8 @@ extern "C" int basd_backward_dots(const basd_shape* shape, const basd_inputs* in
                                      thi, tlo, s.P * s.B, L.Nk, s.Dt, dtm, dtm_lo, st)));
     float* gw = reinterpret_cast<float*>(ws + L.gw);
     TIMED(13, 3, CK(launch_wgrad_dots(tt, dtm, dtm_lo, reinterpret_cast<float*>(ws + L.gwt), reinterpret_cast<float*>(ws + L.rows), s.Lt, s.P, s.B, s.Nt,
-                         s.Ns, s.Dt, gw, reinterpret_cast<float*>(ws + L.gw_part), st, L.path == kPathTeacherTokens && L.Nk == s.Nt && s.Nt != s.Ns, r.teacher_bs)));
+                         s.Ns, s.Dt, gw, reinterpret_cast<float*>(ws + L.gw_part), st, L.path == kPathTeacherTokens && L.Nk == s.Nt && s.Nt != s.Ns, r.teacher_bs,
+                         r.teacher_lo[0] ? &tt_lo : nullptr)));
     return 0;
 }
 
@@ -569,7 +598,7 @@ extern "C" int basd_backward_finish(const basd_shape* shape, const basd_inputs* 
         if (!grad_student[i]) return fail("null grad_student[%d]", i);
         CK(gemm_student_grad(r.student[i], Ms_rows, s.Ds, ghi + static_cast<size_t>(i) * s.Ds * s.Ds, glo + static_cast<size_t>(i) * s.Ds * s.Ds,
                              reinterpret_cast<float*>(ws + L.gdir) + static_cast<size_t>(i) * MsL * s.Ds, corr + static_cast<size_t>(i) * s.Ds,
-                             grad_geo, scale, grad_student[i], grad_dtype == BASD_DTYPE_BF16, r.student_gap ? s.Ns + 1 : 0, s.Ns, st));
+                             grad_geo, scale, grad_student[i], grad_dtype == BASD_DTYPE_BF16, r.student_gap ? s.Ns + 1 : 0, s.Ns, st, r.student_lo[i]));
     }
     return 0;
 }

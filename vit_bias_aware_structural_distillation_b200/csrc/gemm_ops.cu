@@ -162,6 +162,7 @@ static inline int cdiv(long long a, long long b) { return static_cast<int>((a + 
 //                      A_MN   B_MN   BN   MT NA NB T  alias  stages
 using CfgProject = GemmCfg<false, false, 192, 2, 1, 2, 2, false, 2>;     // 256-row tiles: the split P_t tile (49 KB per k-block) is re-read half as often
 using CfgStudentGrad = GemmCfg<false, false, 192, 1, 1, 2, 2, false, 1>;   // one stage (65 KB), 256 TMEM columns: two CTAs per SM overlap each other
+using CfgStudentGrad3 = GemmCfg<false, false, 192, 1, 2, 2, 3, false, 1>;  // split-bf16 students: + S_lo Gamma'_hi (one 81 KB stage)
 using CfgGram    = GemmCfg<true,  true,  192, 2, 1, 1, 1, false, 3>;
 using CfgGramA   = GemmCfg<true,  true,  192, 2, 1, 1, 1, true,  3>;      // D_s <= 192 (one output tile): the B tile is the A tile, one load per k-block
 using CfgGram3   = GemmCfg<true,  true,  192, 2, 2, 2, 3, false, 2>;      // split operands: hi*hi + hi*lo + lo*hi
@@ -190,11 +191,14 @@ static bool f32_tma_ok(const float* out, int ld, long long batch_stride) {
 // TMA stores (ROWMAJOR epilogue; the rows between the samples of a CLS-stripped view are written as zeros).  The one-tile-per-CTA
 // kernel below ran a two-stage ring and per-lane 32-byte row stores with nothing overlapped: 59 k cycles per 256-row tile against
 // 18 k of MMAs (0.48 ms at cfg2).
-static cudaError_t project_persistent(const void* const* X, int n_layers, size_t M, int Dt, const __nv_bfloat16* Phi, const __nv_bfloat16* Plo,
-                                      int Ds, __nv_bfloat16* Z, __nv_bfloat16* Zlo, int gap_period, int gap_valid, cudaStream_t st) {
+// Split-bf16 teachers (Xlo non-null; X[0] = the hi block [n_layers][M][Dt], Xlo the lo block, both packed): the layers are one
+// batched tensor map per half and the third term X_lo P_hi^T joins the two (a_single = 0).
+static cudaError_t project_persistent(const void* const* X, const __nv_bfloat16* Xlo, int n_layers, size_t M, int Dt, const __nv_bfloat16* Phi,
+                                      const __nv_bfloat16* Plo, int Ds, __nv_bfloat16* Z, __nv_bfloat16* Zlo, int gap_period, int gap_valid,
+                                      cudaStream_t st) {
     PolarGemmArgs a;
     memset(&a, 0, sizeof a);
-    a.epi = PG_EPI_ROWMAJOR; a.scale_c = 1.f; a.a_rm = 1; a.b_rm = 1; a.a_single = 1; a.b_shared = 1;
+    a.epi = PG_EPI_ROWMAJOR; a.scale_c = 1.f; a.a_rm = 1; a.b_rm = 1; a.a_single = Xlo ? 0 : 1; a.b_shared = 1;
     a.gap_period = gap_period; a.gap_valid = gap_valid;
     a.ld_out = Ds; a.out_stride = static_cast<long long>(M) * Ds;
     a.m_rows = static_cast<int>(M); a.n_cols = Ds; a.k_total = Dt;
@@ -207,13 +211,36 @@ static cudaError_t project_persistent(const void* const* X, int n_layers, size_t
         a.n_nt = (Ds + a.bn_mma - 1) / a.bn_mma;
     }
     a.b_groups = (a.bn_mma + 63) / 64;
-    const int stage_bytes = 16384 + 2 * a.bn_mma * 128;
+    const int stage_bytes = (Xlo ? 2 : 1) * 16384 + 2 * a.bn_mma * 128;
     const int kTail = 1024 /*alignment*/ + 1024 /*barriers*/ + 4 * 8192 /*epilogue staging*/;
     int stages = (232448 - kTail) / stage_bytes;
     if (stages > 4) stages = 4;
     if (stages < 1) return cudaErrorInvalidValue;
     a.stages = stages;
     const int smem = stages * stage_bytes + kTail;
+    const int sm_count = device_sm_count();
+    if (Xlo) {
+        PolarGemmMaps maps;
+        memset(&maps, 0, sizeof maps);
+        if (make_map(&maps.a[0], X[0], Dt, M, n_layers, Dt, M * Dt, 64)) return cudaErrorInvalidValue;
+        if (make_map(&maps.a[1], Xlo, Dt, M, n_layers, Dt, M * Dt, 64)) return cudaErrorInvalidValue;
+        if (make_map(&maps.b[0], Phi, Dt, Ds, 1, Dt, static_cast<uint64_t>(Ds) * Dt, a.bn_mma)) return cudaErrorInvalidValue;
+        if (make_map(&maps.b[1], Plo, Dt, Ds, 1, Dt, static_cast<uint64_t>(Ds) * Dt, a.bn_mma)) return cudaErrorInvalidValue;
+        a.out_hi = Z; a.out_lo = Zlo;
+        if (make_map(&maps.o[0], Z, Ds, M, n_layers, Ds, M * Ds, 32)) return cudaErrorInvalidValue;
+        if (make_map(&maps.o[1], Zlo, Ds, M, n_layers, Ds, M * Ds, 32)) return cudaErrorInvalidValue;
+        a.n_items = n_layers * a.n_mt * a.n_nt; a.n_batches = n_layers;
+        auto kern = polar_gemm_kernel<false, 4>;
+        static bool configured_split[kMaxDevices] = {};
+        const int dev = current_device();
+        if (!configured_split[dev]) {
+            cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448);
+            if (e != cudaSuccess) return e;
+            configured_split[dev] = true;
+        }
+        kern<<<a.n_items < sm_count ? a.n_items : sm_count, PG_THREADS, smem, st>>>(maps, a);
+        return cudaGetLastError();
+    }
     auto kern = polar_gemm_kernel<false, 4, true>;
     static bool configured[kMaxDevices] = {};
     const int dev = current_device();
@@ -222,7 +249,6 @@ static cudaError_t project_persistent(const void* const* X, int n_layers, size_t
         if (e != cudaSuccess) return e;
         configured[dev] = true;
     }
-    const int sm_count = device_sm_count();
     for (int j0 = 0; j0 < n_layers; j0 += PG_MAX_A_TABLE) {
         const int nl = n_layers - j0 < PG_MAX_A_TABLE ? n_layers - j0 : PG_MAX_A_TABLE;
         PolarGemmMapsT maps;
@@ -246,9 +272,17 @@ static cudaError_t project_persistent(const void* const* X, int n_layers, size_t
 static bool project_use_tile_kernel() { static const bool v = [] { const char* e = getenv("BASD_PROJECT_TILE"); return e && atoi(e) != 0; }(); return v; }
 
 cudaError_t gemm_project(const void* const* X, int n_layers, size_t M, int Dt, const __nv_bfloat16* Phi, const __nv_bfloat16* Plo, int Ds,
-                         __nv_bfloat16* Z, __nv_bfloat16* Zlo, int gap_period, int gap_valid, cudaStream_t st) {
-    if (Ds % 8 == 0 && Dt % 8 == 0 && M < (size_t(1) << 31) - 128 && !project_use_tile_kernel())
-        return project_persistent(X, n_layers, M, Dt, Phi, Plo, Ds, Z, Zlo, gap_period, gap_valid, st);
+                         __nv_bfloat16* Z, __nv_bfloat16* Zlo, int gap_period, int gap_valid, cudaStream_t st, const __nv_bfloat16* Xlo) {
+    const bool persistent_ok = Ds % 8 == 0 && Dt % 8 == 0 && M < (size_t(1) << 31) - 128;
+    if (Xlo) {                              // split-bf16 teachers: the persistent kernel only (the tile kernel has no X_lo term)
+        if (!persistent_ok || gap_period) {
+            snprintf(g_gemm_err, sizeof g_gemm_err, "project: split-bf16 teachers need dense packed layers, Ds, Dt multiples of 8");
+            return cudaErrorInvalidValue;
+        }
+        return project_persistent(X, Xlo, n_layers, M, Dt, Phi, Plo, Ds, Z, Zlo, 0, 0, st);
+    }
+    if (persistent_ok && !project_use_tile_kernel())
+        return project_persistent(X, nullptr, n_layers, M, Dt, Phi, Plo, Ds, Z, Zlo, gap_period, gap_valid, st);
     GemmArgs a;
     memset(&a, 0, sizeof a);
     a.gap_period = gap_period; a.gap_valid = gap_valid;
@@ -615,14 +649,15 @@ static cudaError_t student_grad_persistent(const __nv_bfloat16* S, size_t M, int
 
 cudaError_t gemm_student_grad(const __nv_bfloat16* S, size_t M, int Ds, const __nv_bfloat16* Ghi, const __nv_bfloat16* Glo,
                               const float* gdir, const float* corr, const float* scale_ptr, float scale_host, void* out,
-                              int out_is_bf16, int gap_period, int gap_valid, cudaStream_t st) {
-    // dense bf16 students with a bf16 gradient (the training configuration): persistent kernel; CLS-stripped views (gapped rows)
-    // and fp32 gradients keep the one-tile-per-CTA kernel below
-    if (!gap_period && out_is_bf16 && Ds % 8 == 0 && M < (size_t(1) << 31) - 128)
+                              int out_is_bf16, int gap_period, int gap_valid, cudaStream_t st, const __nv_bfloat16* S_lo) {
+    // dense bf16 students with a bf16 gradient (the training configuration): persistent kernel; CLS-stripped views (gapped rows),
+    // fp32 gradients and split-bf16 students (three terms) keep the one-tile-per-CTA kernel below
+    if (!S_lo && !gap_period && out_is_bf16 && Ds % 8 == 0 && M < (size_t(1) << 31) - 128)
         return student_grad_persistent(S, M, Ds, Ghi, Glo, gdir, corr, scale_ptr, scale_host, static_cast<__nv_bfloat16*>(out), st);
     GemmMaps maps;
     memset(&maps, 0, sizeof maps);
     if (make_map(&maps.a[0], S, Ds, M, 1, Ds, M * Ds, 128)) return cudaErrorInvalidValue;
+    if (S_lo && make_map(&maps.a[1], S_lo, Ds, M, 1, Ds, M * Ds, 128)) return cudaErrorInvalidValue;
     if (make_map(&maps.b[0], Ghi, Ds, Ds, 1, Ds, static_cast<uint64_t>(Ds) * Ds, CfgStudentGrad::kBN)) return cudaErrorInvalidValue;
     if (make_map(&maps.b[1], Glo, Ds, Ds, 1, Ds, static_cast<uint64_t>(Ds) * Ds, CfgStudentGrad::kBN)) return cudaErrorInvalidValue;
     GemmArgs a;
@@ -631,6 +666,8 @@ cudaError_t gemm_student_grad(const __nv_bfloat16* S, size_t M, int Ds, const __
     a.out = out; a.ld_out = Ds; a.rows_valid = static_cast<int>(M); a.cols_valid = Ds;
     a.aux0 = gdir; a.aux1 = corr; a.aux2 = scale_ptr; a.alpha = scale_host; a.beta = out_is_bf16 ? 1.f : 0.f;
     a.gap_period = gap_period; a.gap_valid = gap_valid;
+    static_assert(CfgStudentGrad3::kBN == CfgStudentGrad::kBN, "same tiles");
+    if (S_lo) return launch<CfgStudentGrad3, EpiStudentGrad>(maps, a, dim3(cdiv(Ds, CfgStudentGrad::kBN), cdiv(M, 128), 1), st);
     return launch<CfgStudentGrad, EpiStudentGrad>(maps, a, dim3(cdiv(Ds, CfgStudentGrad::kBN), cdiv(M, 128), 1), st);
 }
 

@@ -152,12 +152,37 @@ polar_prep_student_kernel(PolarArgs g) {
 // ------------------------------------------------------------------------------------------------
 // STAGE = false (tiles that do not fit shared memory, e.g. 576 x 384): the same passes read the tokens straight from
 // global memory (L2-resident: 442 KB per problem).
-template <bool STAGE>
-__global__ void __launch_bounds__(kPrepThreads, STAGE ? 2 : 1)
+// SPLIT: split-bf16 students (g.student_lo, dense): every token is read as hi + lo, before the centring; with STAGE the lo tile
+// is staged behind the hi tile.
+// (8 consecutive values of a raw row as fp32: hi + lo for split students)
+template <bool SPLIT>
+__device__ __forceinline__ void prep_ld8(const __nv_bfloat16* raw, const __nv_bfloat16* raw_lo, size_t idx, float* f) {
+    const uint4 v = *reinterpret_cast<const uint4*>(raw + idx);
+    const __nv_bfloat162* h = reinterpret_cast<const __nv_bfloat162*>(&v);
+#pragma unroll
+    for (int e = 0; e < 4; ++e) {
+        const float2 t = __bfloat1622float2(h[e]);
+        f[2 * e] = t.x;
+        f[2 * e + 1] = t.y;
+    }
+    if (SPLIT) {
+        const uint4 u = *reinterpret_cast<const uint4*>(raw_lo + idx);
+        const __nv_bfloat162* l = reinterpret_cast<const __nv_bfloat162*>(&u);
+#pragma unroll
+        for (int e = 0; e < 4; ++e) {
+            const float2 t = __bfloat1622float2(l[e]);
+            f[2 * e] += t.x;
+            f[2 * e + 1] += t.y;
+        }
+    }
+}
+template <bool STAGE, bool SPLIT = false>
+__global__ void __launch_bounds__(kPrepThreads, STAGE && !SPLIT ? 2 : 1)
 polar_prep_student_vec_kernel(PolarArgs g) {
     extern __shared__ __align__(16) uint8_t sm_raw[];
     const int N = g.Ns, D = g.Ds, pitch = STAGE ? D + 8 : D, oct = D / 8;      // pitch in bf16: rows stay 16-byte aligned
-    float* a_s = reinterpret_cast<float*>(sm_raw + (STAGE ? ((static_cast<size_t>(N) * pitch * 2 + 15) & ~size_t(15)) : 0));
+    const size_t tile_bytes = STAGE ? ((static_cast<size_t>(N) * pitch * 2 + 15) & ~size_t(15)) : 0;
+    float* a_s = reinterpret_cast<float*>(sm_raw + (SPLIT ? 2 : 1) * tile_bytes);
     float* q_s = a_s + N;
     float* mu = q_s + N;                                            // [D]
     float* red = mu + D;                                            // 40
@@ -165,7 +190,9 @@ polar_prep_student_vec_kernel(PolarArgs g) {
     const int prob = blockIdx.x;
     const int i = prob / g.B, b = prob % g.B;
     const __nv_bfloat16* S = g.student[i] + static_cast<size_t>(b) * g.student_bs;
+    const __nv_bfloat16* S_lo = SPLIT ? g.student_lo[i] + static_cast<size_t>(b) * g.student_bs : nullptr;
     const __nv_bfloat16* raw = STAGE ? reinterpret_cast<const __nv_bfloat16*>(sm_raw) : S;      // [N][pitch]
+    const __nv_bfloat16* raw_lo = STAGE ? reinterpret_cast<const __nv_bfloat16*>(sm_raw + tile_bytes) : S_lo;
     for (int n = threadIdx.x; n < N; n += blockDim.x) {
         const float a = g.a[static_cast<size_t>(prob) * N + n];
         a_s[n] = a;
@@ -176,6 +203,8 @@ polar_prep_student_vec_kernel(PolarArgs g) {
         for (int t = threadIdx.x; t < N * oct; t += blockDim.x) {
             const int n = t / oct, o = t - n * oct;
             *reinterpret_cast<uint4*>(stage + n * pitch + o * 8) = *reinterpret_cast<const uint4*>(S + static_cast<size_t>(n) * D + o * 8);
+            if (SPLIT)
+                *reinterpret_cast<uint4*>(stage + tile_bytes / 2 + n * pitch + o * 8) = *reinterpret_cast<const uint4*>(S_lo + static_cast<size_t>(n) * D + o * 8);
         }
     }
     __syncthreads();
@@ -186,15 +215,11 @@ polar_prep_student_vec_kernel(PolarArgs g) {
         if (sl < slices) {
             float m[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
             for (int n = sl; n < N; n += slices) {
-                const uint4 v = *reinterpret_cast<const uint4*>(raw + n * pitch + o * 8);
-                const __nv_bfloat162* h = reinterpret_cast<const __nv_bfloat162*>(&v);
+                float f[8];
+                prep_ld8<SPLIT>(raw, raw_lo, static_cast<size_t>(n) * pitch + o * 8, f);
                 const float an = a_s[n];
 #pragma unroll
-                for (int e = 0; e < 4; ++e) {
-                    const float2 f = __bfloat1622float2(h[e]);
-                    m[2 * e] = fmaf(an, f.x, m[2 * e]);
-                    m[2 * e + 1] = fmaf(an, f.y, m[2 * e + 1]);
-                }
+                for (int e = 0; e < 8; ++e) m[e] = fmaf(an, f[e], m[e]);
             }
 #pragma unroll
             for (int e = 0; e < 8; ++e) partial[sl * D + o * 8 + e] = m[e];
@@ -215,12 +240,11 @@ polar_prep_student_vec_kernel(PolarArgs g) {
         float s = 0.f;
         const float qn = q_s[n];
         for (int o = lane; o < oct; o += 32) {
-            const uint4 v = *reinterpret_cast<const uint4*>(raw + n * pitch + o * 8);
-            const __nv_bfloat162* h = reinterpret_cast<const __nv_bfloat162*>(&v);
+            float f[8];
+            prep_ld8<SPLIT>(raw, raw_lo, static_cast<size_t>(n) * pitch + o * 8, f);
 #pragma unroll
             for (int e = 0; e < 4; ++e) {
-                const float2 f = __bfloat1622float2(h[e]);
-                const float x = qn * (f.x - mu[o * 8 + 2 * e]), y = qn * (f.y - mu[o * 8 + 2 * e + 1]);
+                const float x = qn * (f[2 * e] - mu[o * 8 + 2 * e]), y = qn * (f[2 * e + 1] - mu[o * 8 + 2 * e + 1]);
                 s = fmaf(x, x, fmaf(y, y, s));
             }
         }
@@ -238,15 +262,11 @@ polar_prep_student_vec_kernel(PolarArgs g) {
         const int d0 = cb * 64 + j0;
         float v[8];
         if (d0 < D) {
-            const uint4 r = *reinterpret_cast<const uint4*>(raw + n * pitch + d0);
-            const __nv_bfloat162* h = reinterpret_cast<const __nv_bfloat162*>(&r);
+            float f[8];
+            prep_ld8<SPLIT>(raw, raw_lo, static_cast<size_t>(n) * pitch + d0, f);
             const float qn = q_s[n];
 #pragma unroll
-            for (int e = 0; e < 4; ++e) {
-                const float2 f = __bfloat1622float2(h[e]);
-                v[2 * e] = qn * (f.x - mu[d0 + 2 * e]);
-                v[2 * e + 1] = qn * (f.y - mu[d0 + 2 * e + 1]);
-            }
+            for (int e = 0; e < 8; ++e) v[e] = qn * (f[e] - mu[d0 + e]);
         } else {
 #pragma unroll
             for (int e = 0; e < 8; ++e) v[e] = 0.f;
@@ -269,7 +289,12 @@ polar_prep_student_vec_kernel(PolarArgs g) {
 #pragma unroll
         for (int e = 0; e < 8; ++e) {
             const int n = nb * 64 + j0 + e;
-            v[e] = n < N ? q_s[n] * (__bfloat162float(raw[n * pitch + d]) - md) : 0.f;
+            float x = 0.f;
+            if (n < N) {
+                x = __bfloat162float(raw[n * pitch + d]);
+                if (SPLIT) x += __bfloat162float(raw_lo[n * pitch + d]);
+            }
+            v[e] = n < N ? q_s[n] * (x - md) : 0.f;
         }
         store_split8(wh, wl, (static_cast<size_t>(nb) * D + d) * 64 + j0, v);
     }
@@ -731,23 +756,36 @@ long long* polar_dbg_ptr(int which) { long long* p = nullptr; cudaGetSymbolAddre
 
 #define PCK(expr) do { cudaError_t _e = (expr); if (_e != cudaSuccess) return _e; } while (0)
 
+// prep_student for D_s % 8 == 0 (both polar forms): the raw token tile is staged in shared memory when it fits (split-bf16
+// students stage their lo tile too), otherwise read from global memory
+template <bool SPLIT>
+static cudaError_t launch_prep_student_vec(const PolarArgs& g, cudaStream_t st) {
+    const int N = g.Ns, D = g.Ds, nprob = g.n_problems;
+    const int slices = kPrepThreads / (D / 8);
+    const size_t small = (2 * N + D + 40 + static_cast<size_t>(slices) * D) * sizeof(float);
+    const size_t smem = (SPLIT ? 2 : 1) * ((static_cast<size_t>(N) * (D + 8) * 2 + 15) & ~size_t(15)) + small;
+    if (smem <= 227 * 1024) {
+        PCK(cudaFuncSetAttribute(polar_prep_student_vec_kernel<true, SPLIT>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
+        polar_prep_student_vec_kernel<true, SPLIT><<<nprob, kPrepThreads, smem, st>>>(g);
+    } else {
+        PCK(cudaFuncSetAttribute(polar_prep_student_vec_kernel<false, SPLIT>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(small)));
+        polar_prep_student_vec_kernel<false, SPLIT><<<nprob, kPrepThreads, small, st>>>(g);
+    }
+    return cudaGetLastError();
+}
+static cudaError_t launch_prep_student_vec(const PolarArgs& g, cudaStream_t st) {
+    return g.student_lo[0] ? launch_prep_student_vec<true>(g, st) : launch_prep_student_vec<false>(g, st);
+}
+
 cudaError_t launch_polar_procrustes(const PolarArgs& g, cudaStream_t st, int* launches) {
     const int N = g.Ns, D = g.Ds, nprob = g.n_problems;
     int count = 0;
     {
         TimingScope ts(kSlotPolarPrep, st, 2);
         if (D % 8 == 0) {
-            const int slices = kPrepThreads / (D / 8);
-            const size_t small = (2 * N + D + 40 + static_cast<size_t>(slices) * D) * sizeof(float);
-            const size_t smem = ((static_cast<size_t>(N) * (D + 8) * 2 + 15) & ~size_t(15)) + small;
-            if (smem <= 227 * 1024) {
-                PCK(cudaFuncSetAttribute(polar_prep_student_vec_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
-                polar_prep_student_vec_kernel<true><<<nprob, kPrepThreads, smem, st>>>(g);
-            } else {
-                PCK(cudaFuncSetAttribute(polar_prep_student_vec_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(small)));
-                polar_prep_student_vec_kernel<false><<<nprob, kPrepThreads, small, st>>>(g);
-            }
+            PCK(launch_prep_student_vec(g, st));
         } else {
+            if (g.student_lo[0]) return cudaErrorInvalidValue;      // (check_shape requires D_s % 8 == 0)
             const size_t smem = (static_cast<size_t>(N) * (D + 1) + 2 * N + D + 64) * sizeof(float);
             PCK(cudaFuncSetAttribute(polar_prep_student_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
             polar_prep_student_kernel<<<nprob, kPrepThreads, smem, st>>>(g);
@@ -867,17 +905,7 @@ cudaError_t launch_polar_procrustes_vt(const PolarArgs& g, cudaStream_t st, int*
     {
         TimingScope ts(kSlotPolarPrep, st, 3);
         if (D % 8 != 0) return cudaErrorInvalidValue;
-        const int slices = kPrepThreads / (D / 8);
-        const size_t small = (2 * N + D + 40 + static_cast<size_t>(slices) * D) * sizeof(float);
-        const size_t smem = ((static_cast<size_t>(N) * (D + 8) * 2 + 15) & ~size_t(15)) + small;
-        if (smem <= 227 * 1024) {
-            PCK(cudaFuncSetAttribute(polar_prep_student_vec_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
-            polar_prep_student_vec_kernel<true><<<nprob, kPrepThreads, smem, st>>>(g);
-        } else {
-            PCK(cudaFuncSetAttribute(polar_prep_student_vec_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(small)));
-            polar_prep_student_vec_kernel<false><<<nprob, kPrepThreads, small, st>>>(g);
-        }
-        PCK(cudaGetLastError());
+        PCK(launch_prep_student_vec(g, st));
         const int ld = (M + 3) & ~3;
         const size_t smem_t = (static_cast<size_t>(ld) * M + 2 * N + 3 * M + 64) * sizeof(float);
         PCK(cudaFuncSetAttribute(vt_prep_teacher_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem_t)));

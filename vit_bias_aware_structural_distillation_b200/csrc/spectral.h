@@ -62,14 +62,17 @@ cudaError_t launch_colsum(const ColsumJobs& jobs, int n_jobs, size_t rows, int D
                           long long batch_stride = 0);
 cudaError_t launch_importance_mix(const float* rows, const float* w, int Lt, int P, int B, int Nt, int Ns, float* a,
                                   float* ssum, cudaStream_t st);
+// teacher_lo (non-null): split-bf16 teacher tokens, read as hi + lo (BASD_DTYPE_F32_SPLIT)
 cudaError_t launch_mix_teacher(const PtrTable& teacher, const float* w, int Lt, int P, int B, int Nt, int Ns, int Dt,
-                               __nv_bfloat16* hi, __nv_bfloat16* lo, cudaStream_t st, long long teacher_batch_stride = 0 /*0: Nt * Dt*/);
+                               __nv_bfloat16* hi, __nv_bfloat16* lo, cudaStream_t st, long long teacher_batch_stride = 0 /*0: Nt * Dt*/,
+                               const PtrTable* teacher_lo = nullptr);
 // Dtm is [P][B][Nd][Dt] with Nd = Ns (gradient w.r.t. the token-aligned mixed teacher) or, with dtm_unaligned, Nd = Nt
 // (gradient w.r.t. the mixed teacher on its own token grid: no resampling in the dots)
 cudaError_t launch_wgrad_dots(const PtrTable& teacher, const __nv_bfloat16* Dtm, const __nv_bfloat16* Dtm_lo, const float* gwt, const float* rows,
                               int Lt, int P, int B, int Nt, int Ns, int Dt, float* gw /*[P][Lt]*/,
                               float* gw_part /*wgrad_part_floats(P, Lt) floats: per-CTA partials, summed in a fixed order*/,
-                              cudaStream_t st, bool dtm_unaligned = false, long long teacher_batch_stride = 0 /*0: Nt * Dt*/);
+                              cudaStream_t st, bool dtm_unaligned = false, long long teacher_batch_stride = 0 /*0: Nt * Dt*/,
+                              const PtrTable* teacher_lo = nullptr /*split-bf16 teachers: read as hi + lo*/);
 size_t wgrad_part_floats(int P, int Lt);
 cudaError_t launch_cls_attention_rows(const void* q, const void* k, int is_bf16, int B, int H, int S, int dh,
                                       const long long* q_strides /*[b,h]*/, const long long* k_strides /*[b,h,s]*/, float scale,
@@ -93,8 +96,10 @@ int gemm_init_driver_api();               // resolves cuTensorMapEncodeTiled; 0 
 // Z[j] = X[j] P^T for n_layers separate [M][Dt] bf16 tensors; Zhi / Zlo are [n_layers][M][Ds]
 // gap_period > 0: rows r of X with r % gap_period >= gap_valid lie between two samples (CLS-stripped view of a
 // [B][N+1][Dt] buffer read as a dense matrix of M rows): their Z rows are written as zeros
+// Xlo non-null (split-bf16 teachers): X[0] is the hi block [n_layers][M][Dt], Xlo the lo block; Z = X_hi P_hi^T + X_hi P_lo^T + X_lo P_hi^T
 cudaError_t gemm_project(const void* const* X, int n_layers, size_t M, int Dt, const __nv_bfloat16* Phi, const __nv_bfloat16* Plo,
-                         int Ds, __nv_bfloat16* Zhi, __nv_bfloat16* Zlo, int gap_period, int gap_valid, cudaStream_t st);
+                         int Ds, __nv_bfloat16* Zhi, __nv_bfloat16* Zlo, int gap_period, int gap_valid, cudaStream_t st,
+                         const __nv_bfloat16* Xlo = nullptr);
 // Zlo may be null (exact bf16 input); otherwise Z = Zhi + Zlo and the Gram uses hi*hi + hi*lo + lo*hi
 // G[i] (stride g_stride floats) += S_i^T S_i for n separate exact-bf16 [M][Ds] tensors, one launch
 // Split-K slices go to `part` (gemm_gram_part_floats floats) and are summed in a fixed order: bitwise repeatable Grams.
@@ -114,7 +119,8 @@ cudaError_t gemm_theta_apply(const __nv_bfloat16* theta_hi, const __nv_bfloat16*
                              const __nv_bfloat16* Tlo, int batches, int Ns, int Dt, __nv_bfloat16* Dtm, __nv_bfloat16* Dtm_lo, cudaStream_t st);
 cudaError_t gemm_student_grad(const __nv_bfloat16* S, size_t M, int Ds, const __nv_bfloat16* Ghi, const __nv_bfloat16* Glo,
                               const float* gdir, const float* corr, const float* scale_ptr, float scale_host, void* out,
-                              int out_is_bf16, int gap_period, int gap_valid, cudaStream_t st);
+                              int out_is_bf16, int gap_period, int gap_valid, cudaStream_t st,
+                              const __nv_bfloat16* S_lo = nullptr /*split-bf16 students: adds the term S_lo Gamma'_hi*/);
 // generic test hook: C[M][N] (fp32) = A[M][K] * B[N][K]^T or with MN-major operands (see basd_b200.h selftest)
 cudaError_t gemm_selftest(int variant, const __nv_bfloat16* A, const __nv_bfloat16* B, float* C, int M, int N, int K,
                           cudaStream_t st);
@@ -174,6 +180,7 @@ struct PolarArgs {
     float* thraw;                         // [P*B][Nt][Nt]
     float* ftf;                           // [P*B][Nt][Nt]   F^T F
     const __nv_bfloat16* student[kMaxPoints];   // [B][Ns][Ds] bf16, batch stride student_bs elements (Ns * Ds when dense)
+    const __nv_bfloat16* student_lo[kMaxPoints];  // split-bf16 students: lo halves (dense), s = hi + lo; null otherwise
     long long student_bs;
     const float* Ktt;                     // [P*B][Ns][Ns]   uncentred token Gram of the mixed teacher
     const float* a;                       // [P*B][Ns]       normalised importance

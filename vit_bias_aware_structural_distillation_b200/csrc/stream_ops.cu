@@ -23,6 +23,13 @@ __device__ __forceinline__ void bf16x8_to_float(const uint4& v, float* f) {
         f[2 * i + 1] = t.y;
     }
 }
+// f[i] += the eight bf16 of v (the lo half of a split-bf16 pair onto its hi half)
+__device__ __forceinline__ void add_bf16x8(const uint4& v, float* f) {
+    float l[8];
+    bf16x8_to_float(v, l);
+#pragma unroll
+    for (int i = 0; i < 8; ++i) f[i] += l[i];
+}
 __device__ __forceinline__ uint32_t pack2(float a, float b) {
     __nv_bfloat162 v = __floats2bfloat162_rn(a, b);
     return *reinterpret_cast<uint32_t*>(&v);
@@ -285,12 +292,14 @@ cudaError_t launch_importance_mix(const float* rows, const float* w, int Lt, int
 // Tbar[i][b][n][:] = sum_j w[i][j] * interp(T_j[b])[n][:]  -> bf16 hi + lo.  One thread = one 8-wide vector.
 // Teacher vectors are loaded twelve layers at a time before the first use (one load and its use alternating per layer left
 // one request in flight per thread: 4.0 TB/s; six at a time 4.6, twelve 5.1), 32-bit index arithmetic, no interpolation
-// branch when N_t == N_s.
+// branch when N_t == N_s.  TSPLIT: split-bf16 teacher tokens (teacher_lo holds the lo halves, same layout), read as hi + lo;
+// six layers at a time so that the doubled loads stay in registers.
 constexpr int MT_JC = 12;
-template <int PMAX, bool INTERP>
+template <int PMAX, bool INTERP, bool TSPLIT = false>
 __global__ void __launch_bounds__(256)
 mix_teacher_kernel(PtrTable teacher, const float* __restrict__ w, int Lt, int P, int B, int Nt, int Ns, int Dt, long long tbs,
-                   __nv_bfloat16* __restrict__ hi, __nv_bfloat16* __restrict__ lo) {
+                   __nv_bfloat16* __restrict__ hi, __nv_bfloat16* __restrict__ lo, PtrTable teacher_lo) {
+    constexpr int JC = TSPLIT ? MT_JC / 2 : MT_JC;
     __shared__ float ws[PMAX * kMaxLayers];
     for (int t = threadIdx.x; t < P * Lt; t += blockDim.x) ws[t] = w[t];
     __syncthreads();
@@ -307,23 +316,31 @@ mix_teacher_kernel(PtrTable teacher, const float* __restrict__ w, int Lt, int P,
         for (int i = 0; i < PMAX; ++i)
 #pragma unroll
             for (int e = 0; e < 8; ++e) acc[i][e] = 0.f;
-        for (int j0 = 0; j0 < Lt; j0 += MT_JC) {
-            uint4 t0[MT_JC], t1[INTERP ? MT_JC : 1];
+        for (int j0 = 0; j0 < Lt; j0 += JC) {
+            uint4 t0[JC], t1[INTERP ? JC : 1], u0[TSPLIT ? JC : 1], u1[TSPLIT && INTERP ? JC : 1];
 #pragma unroll
-            for (int jj = 0; jj < MT_JC; ++jj) {
+            for (int jj = 0; jj < JC; ++jj) {
                 const bool ok = j0 + jj < Lt;
-                const __nv_bfloat16* T = reinterpret_cast<const __nv_bfloat16*>(teacher.p[ok ? j0 + jj : 0]) + static_cast<size_t>(b) * tbs + dv * 8;
+                const size_t boff = static_cast<size_t>(b) * tbs + dv * 8;
+                const __nv_bfloat16* T = reinterpret_cast<const __nv_bfloat16*>(teacher.p[ok ? j0 + jj : 0]) + boff;
                 t0[jj] = ok ? ld_nc_16(T + static_cast<size_t>(i0) * Dt) : zero4;
                 if (INTERP) t1[jj] = ok ? ld_nc_16(T + static_cast<size_t>(i1) * Dt) : zero4;
+                if (TSPLIT) {
+                    const __nv_bfloat16* U = reinterpret_cast<const __nv_bfloat16*>(teacher_lo.p[ok ? j0 + jj : 0]) + boff;
+                    u0[jj] = ok ? ld_nc_16(U + static_cast<size_t>(i0) * Dt) : zero4;
+                    if (INTERP) u1[jj] = ok ? ld_nc_16(U + static_cast<size_t>(i1) * Dt) : zero4;
+                }
             }
 #pragma unroll
-            for (int jj = 0; jj < MT_JC; ++jj) {
+            for (int jj = 0; jj < JC; ++jj) {
                 if (j0 + jj < Lt) {
                     float f[8];
                     bf16x8_to_float(t0[jj], f);
+                    if (TSPLIT) add_bf16x8(u0[jj], f);
                     if (INTERP) {
                         float g[8];
                         bf16x8_to_float(t1[jj], g);
+                        if (TSPLIT) add_bf16x8(u1[jj], g);
 #pragma unroll
                         for (int e = 0; e < 8; ++e) f[e] = (1.f - lam) * f[e] + lam * g[e];
                     }
@@ -362,20 +379,23 @@ mix_teacher_kernel(PtrTable teacher, const float* __restrict__ w, int Lt, int P,
     }
 }
 cudaError_t launch_mix_teacher(const PtrTable& teacher, const float* w, int Lt, int P, int B, int Nt, int Ns, int Dt,
-                               __nv_bfloat16* hi, __nv_bfloat16* lo, cudaStream_t st, long long tbs) {
+                               __nv_bfloat16* hi, __nv_bfloat16* lo, cudaStream_t st, long long tbs, const PtrTable* teacher_lo) {
     if (tbs <= 0) tbs = static_cast<long long>(Nt) * Dt;
     if (Dt % 8 != 0 || P > kMaxPoints) return cudaErrorInvalidValue;
     const size_t total = static_cast<size_t>(B) * Ns * (Dt / 8);
     const int blocks = static_cast<int>((total + 255) / 256 < 148 * 8 ? (total + 255) / 256 : 148 * 8);
     if (static_cast<unsigned long long>(B) * Ns * (Dt / 8) >= (1ull << 32)) return cudaErrorInvalidValue;
     const bool interp = Nt != Ns;
-    if (P <= 4) {
-        if (interp) mix_teacher_kernel<4, true><<<blocks, 256, 0, st>>>(teacher, w, Lt, P, B, Nt, Ns, Dt, tbs, hi, lo);
-        else mix_teacher_kernel<4, false><<<blocks, 256, 0, st>>>(teacher, w, Lt, P, B, Nt, Ns, Dt, tbs, hi, lo);
+    const PtrTable tl = teacher_lo ? *teacher_lo : PtrTable{};
+#define MIX_LAUNCH(PM, IN, SP) mix_teacher_kernel<PM, IN, SP><<<blocks, 256, 0, st>>>(teacher, w, Lt, P, B, Nt, Ns, Dt, tbs, hi, lo, tl)
+    if (teacher_lo) {
+        if (P <= 4) { if (interp) MIX_LAUNCH(4, true, true); else MIX_LAUNCH(4, false, true); }
+        else { if (interp) MIX_LAUNCH(8, true, true); else MIX_LAUNCH(8, false, true); }
     } else {
-        if (interp) mix_teacher_kernel<8, true><<<blocks, 256, 0, st>>>(teacher, w, Lt, P, B, Nt, Ns, Dt, tbs, hi, lo);
-        else mix_teacher_kernel<8, false><<<blocks, 256, 0, st>>>(teacher, w, Lt, P, B, Nt, Ns, Dt, tbs, hi, lo);
+        if (P <= 4) { if (interp) MIX_LAUNCH(4, true, false); else MIX_LAUNCH(4, false, false); }
+        else { if (interp) MIX_LAUNCH(8, true, false); else MIX_LAUNCH(8, false, false); }
     }
+#undef MIX_LAUNCH
     return cudaGetLastError();
 }
 
@@ -385,18 +405,20 @@ constexpr int WG_PC = 4, WG_JC = 12;
 // All 16-byte loads of a position (WG_PC gradient vectors, WG_JC teacher vectors, twice that when interpolating) are issued
 // before the first use: with a load and its use alternating per layer the kernel ran at 2 TB/s, one L2/HBM latency per layer.
 // Every CTA writes its WG_PC x WG_JC partial dots to gw_part[blockIdx.x][P][Lt]; wgrad_reduce_kernel adds the CTAs (and the
-// importance partials) in a fixed order.
-template <bool INTERP, bool SPLIT>
+// importance partials) in a fixed order.  TSPLIT: split-bf16 teacher tokens read as hi + lo, six layers per CTA.
+template <bool TSPLIT> __host__ __device__ constexpr int wgrad_jc() { return TSPLIT ? WG_JC / 2 : WG_JC; }
+template <bool INTERP, bool SPLIT, bool TSPLIT = false>
 __global__ void __launch_bounds__(256)
 wgrad_dots_kernel(PtrTable teacher, const __nv_bfloat16* __restrict__ Dtm, const __nv_bfloat16* __restrict__ DtmLo, int Lt, int P, int B, int Nt,
-                  int Ns, int Dt, long long tbs, float* __restrict__ gw_part) {
-    const int n_jc = (Lt + WG_JC - 1) / WG_JC;
-    const int i_base = (blockIdx.y / n_jc) * WG_PC, j_base = (blockIdx.y % n_jc) * WG_JC;
-    float acc[WG_PC][WG_JC];
+                  int Ns, int Dt, long long tbs, float* __restrict__ gw_part, PtrTable teacher_lo) {
+    constexpr int JC = wgrad_jc<TSPLIT>();
+    const int n_jc = (Lt + JC - 1) / JC;
+    const int i_base = (blockIdx.y / n_jc) * WG_PC, j_base = (blockIdx.y % n_jc) * JC;
+    float acc[WG_PC][JC];
 #pragma unroll
     for (int i = 0; i < WG_PC; ++i)
 #pragma unroll
-        for (int j = 0; j < WG_JC; ++j) acc[i][j] = 0.f;
+        for (int j = 0; j < JC; ++j) acc[i][j] = 0.f;
     const uint32_t vpr = static_cast<uint32_t>(Dt) / 8u;
     const uint32_t total = static_cast<uint32_t>(B) * Ns * vpr;            // < 2^32 (checked by the launcher)
     const uint4 zero4 = make_uint4(0u, 0u, 0u, 0u);
@@ -405,7 +427,7 @@ wgrad_dots_kernel(PtrTable teacher, const __nv_bfloat16* __restrict__ Dtm, const
         const uint32_t b = row / static_cast<uint32_t>(Ns), n = row - b * Ns;
         int i0, i1; float lam;
         interp_index(static_cast<int>(n), Nt, Ns, i0, i1, lam);
-        uint4 draw[WG_PC], dlow[SPLIT ? WG_PC : 1], t0[WG_JC], t1[INTERP ? WG_JC : 1];
+        uint4 draw[WG_PC], dlow[SPLIT ? WG_PC : 1], t0[JC], t1[INTERP ? JC : 1], u0[TSPLIT ? JC : 1], u1[TSPLIT && INTERP ? JC : 1];
 #pragma unroll
         for (int i = 0; i < WG_PC; ++i) {
             const size_t off = ((static_cast<size_t>(i_base + i < P ? i_base + i : 0) * B + b) * Ns + n) * Dt + dv * 8;
@@ -413,11 +435,17 @@ wgrad_dots_kernel(PtrTable teacher, const __nv_bfloat16* __restrict__ Dtm, const
             if (SPLIT) dlow[i] = i_base + i < P ? ld_nc_16(DtmLo + off) : zero4;
         }
 #pragma unroll
-        for (int j = 0; j < WG_JC; ++j) {
+        for (int j = 0; j < JC; ++j) {
             const bool ok = j_base + j < Lt;
-            const __nv_bfloat16* T = reinterpret_cast<const __nv_bfloat16*>(teacher.p[ok ? j_base + j : 0]) + static_cast<size_t>(b) * tbs + dv * 8;
+            const size_t boff = static_cast<size_t>(b) * tbs + dv * 8;
+            const __nv_bfloat16* T = reinterpret_cast<const __nv_bfloat16*>(teacher.p[ok ? j_base + j : 0]) + boff;
             t0[j] = ok ? ld_nc_16(T + static_cast<size_t>(i0) * Dt) : zero4;
             if (INTERP) t1[j] = ok ? ld_nc_16(T + static_cast<size_t>(i1) * Dt) : zero4;
+            if (TSPLIT) {
+                const __nv_bfloat16* U = reinterpret_cast<const __nv_bfloat16*>(teacher_lo.p[ok ? j_base + j : 0]) + boff;
+                u0[j] = ok ? ld_nc_16(U + static_cast<size_t>(i0) * Dt) : zero4;
+                if (INTERP) u1[j] = ok ? ld_nc_16(U + static_cast<size_t>(i1) * Dt) : zero4;
+            }
         }
         float dtv[WG_PC][8];
 #pragma unroll
@@ -431,12 +459,14 @@ wgrad_dots_kernel(PtrTable teacher, const __nv_bfloat16* __restrict__ Dtm, const
             }
         }
 #pragma unroll
-        for (int j = 0; j < WG_JC; ++j) {
+        for (int j = 0; j < JC; ++j) {
             float f[8];
             bf16x8_to_float(t0[j], f);
+            if (TSPLIT) add_bf16x8(u0[j], f);
             if (INTERP) {
                 float g[8];
                 bf16x8_to_float(t1[j], g);
+                if (TSPLIT) add_bf16x8(u1[j], g);
 #pragma unroll
                 for (int e = 0; e < 8; ++e) f[e] = (1.f - lam) * f[e] + lam * g[e];
             }
@@ -449,17 +479,17 @@ wgrad_dots_kernel(PtrTable teacher, const __nv_bfloat16* __restrict__ Dtm, const
             }
         }
     }
-    __shared__ float red[8][WG_PC * WG_JC];               // one row per warp (256 threads)
+    __shared__ float red[8][WG_PC * JC];                  // one row per warp (256 threads)
 #pragma unroll
     for (int i = 0; i < WG_PC; ++i)
 #pragma unroll
-        for (int j = 0; j < WG_JC; ++j) {
+        for (int j = 0; j < JC; ++j) {
             const float s = warp_sum(acc[i][j]);
-            if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5][i * WG_JC + j] = s;
+            if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5][i * JC + j] = s;
         }
     __syncthreads();
-    for (int t = threadIdx.x; t < WG_PC * WG_JC; t += blockDim.x) {
-        const int i = i_base + t / WG_JC, j = j_base + t % WG_JC;
+    for (int t = threadIdx.x; t < WG_PC * JC; t += blockDim.x) {
+        const int i = i_base + t / JC, j = j_base + t % JC;
         float s = 0.f;
 #pragma unroll
         for (int wv = 0; wv < 8; ++wv) s += red[wv][t];
@@ -500,18 +530,25 @@ wgrad_reduce_kernel(const float* __restrict__ gw_part, int n_part, int PL, float
 constexpr int kWgradDotCtas = 148 * 4, kWgradImpSlices = 16;
 size_t wgrad_part_floats(int P, int Lt) { return static_cast<size_t>(kWgradDotCtas + kWgradImpSlices) * P * Lt; }
 cudaError_t launch_wgrad_dots(const PtrTable& teacher, const __nv_bfloat16* Dtm, const __nv_bfloat16* DtmLo, const float* gwt, const float* rows, int Lt, int P,
-                              int B, int Nt, int Ns, int Dt, float* gw, float* gw_part, cudaStream_t st, bool dtm_unaligned, long long tbs) {
+                              int B, int Nt, int Ns, int Dt, float* gw, float* gw_part, cudaStream_t st, bool dtm_unaligned, long long tbs,
+                              const PtrTable* teacher_lo) {
     if (tbs <= 0) tbs = static_cast<long long>(Nt) * Dt;
     if (Dt % 8 != 0 || static_cast<unsigned long long>(B) * Ns * (Dt / 8) >= (1ull << 32) || !gw_part) return cudaErrorInvalidValue;
-    const int ny = ((P + WG_PC - 1) / WG_PC) * ((Lt + WG_JC - 1) / WG_JC);
+    const int jc = teacher_lo ? wgrad_jc<true>() : wgrad_jc<false>();
+    const int ny = ((P + WG_PC - 1) / WG_PC) * ((Lt + jc - 1) / jc);
     const dim3 grid(kWgradDotCtas, ny);
-    if (Nt == Ns || dtm_unaligned) {
-        if (DtmLo) wgrad_dots_kernel<false, true><<<grid, 256, 0, st>>>(teacher, Dtm, DtmLo, Lt, P, B, Nt, Nt, Dt, tbs, gw_part);
-        else wgrad_dots_kernel<false, false><<<grid, 256, 0, st>>>(teacher, Dtm, DtmLo, Lt, P, B, Nt, Nt, Dt, tbs, gw_part);
+    const PtrTable tl = teacher_lo ? *teacher_lo : PtrTable{};
+    const bool aligned = Nt == Ns || dtm_unaligned;
+    const int ns = aligned ? Nt : Ns;
+#define WG_LAUNCH(IN, SP, TS) wgrad_dots_kernel<IN, SP, TS><<<grid, 256, 0, st>>>(teacher, Dtm, DtmLo, Lt, P, B, Nt, ns, Dt, tbs, gw_part, tl)
+    if (teacher_lo) {
+        if (aligned) { if (DtmLo) WG_LAUNCH(false, true, true); else WG_LAUNCH(false, false, true); }
+        else { if (DtmLo) WG_LAUNCH(true, true, true); else WG_LAUNCH(true, false, true); }
     } else {
-        if (DtmLo) wgrad_dots_kernel<true, true><<<grid, 256, 0, st>>>(teacher, Dtm, DtmLo, Lt, P, B, Nt, Ns, Dt, tbs, gw_part);
-        else wgrad_dots_kernel<true, false><<<grid, 256, 0, st>>>(teacher, Dtm, DtmLo, Lt, P, B, Nt, Ns, Dt, tbs, gw_part);
+        if (aligned) { if (DtmLo) WG_LAUNCH(false, true, false); else WG_LAUNCH(false, false, false); }
+        else { if (DtmLo) WG_LAUNCH(true, true, false); else WG_LAUNCH(true, false, false); }
     }
+#undef WG_LAUNCH
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return e;
     const int slices = B < kWgradImpSlices ? B : kWgradImpSlices;

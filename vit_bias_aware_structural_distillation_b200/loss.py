@@ -26,7 +26,22 @@ import torch.nn as nn
 import torch.nn.functional as F
 
 from . import _lib
-from ._lib import ATTN_QUERY_MEAN, DTYPE_BF16, DTYPE_F32, MODE_LOSS, MODE_PAIR, MODE_SELECTOR, Inputs, Shape
+from ._lib import ATTN_QUERY_MEAN, DTYPE_BF16, DTYPE_F32, DTYPE_F32_SPLIT, MODE_LOSS, MODE_PAIR, MODE_SELECTOR, Inputs, Shape
+
+# How the loss reads fp32 tokens: "bf16" rounds them to bf16 on entry (the default), "fp32" carries them as split-bf16 pairs
+# hi + lo through every kernel that reads them (fp32-class accuracy; DESIGN.md section 8).  bf16 tokens read the same either way.
+TOKEN_PRECISIONS = ("bf16", "fp32")
+
+
+def _check_token_precision(token_precision) -> str:
+    if not isinstance(token_precision, str) or token_precision not in TOKEN_PRECISIONS:
+        raise _lib.BasdError(f"token_precision must be one of {TOKEN_PRECISIONS}, got {token_precision!r}")
+    return token_precision
+
+
+def _split_tokens(students, teachers, token_precision: str) -> bool:
+    """True when the tokens go in as split-bf16 pairs: token_precision "fp32" and any token tensor that is not bf16."""
+    return _check_token_precision(token_precision) == "fp32" and any(t.dtype != torch.bfloat16 for t in list(students) + list(teachers))
 
 
 # --------------------------------------------------------------------------------------------- low-level plumbing
@@ -45,9 +60,11 @@ def _stream_ptr(dev=None) -> int:
 
 def _prepare(students: Sequence[torch.Tensor], teachers: Sequence[torch.Tensor], attns: Sequence[torch.Tensor],
              proj_s: torch.Tensor, proj_t: torch.Tensor, log_temperatures: torch.Tensor, has_cls: bool, world_size: int,
-             polar_steps: int = 0, mode: int = MODE_LOSS):
+             polar_steps: int = 0, mode: int = MODE_LOSS, token_precision: str = "bf16"):
     """Builds the C structs.  Returns (shape, inputs, keepalive) — keepalive holds every tensor whose pointer is used.
-    mode (include/basd_b200.h): MODE_PAIR reads no projections / temperatures, MODE_SELECTOR no attention maps."""
+    mode (include/basd_b200.h): MODE_PAIR reads no projections / temperatures, MODE_SELECTOR no attention maps.
+    token_precision "fp32": if any token tensor is not bf16, all of them go in as fp32 split-bf16 pairs (BASD_DTYPE_F32_SPLIT)."""
+    split = _split_tokens(students, teachers, token_precision)
     if not students or not teachers or (mode != MODE_SELECTOR and len(teachers) != len(attns)):
         raise _lib.BasdError("need >= 1 student tensor, >= 1 teacher tensor and one attention map per teacher layer")
     if mode == MODE_SELECTOR:
@@ -56,7 +73,7 @@ def _prepare(students: Sequence[torch.Tensor], teachers: Sequence[torch.Tensor],
     if dev.type != "cuda":
         raise _lib.BasdError("the BASD loss path runs on a CUDA device only (no CPU fallback); got tensors on " + str(dev))
     act_dt = students[0].dtype
-    if act_dt not in (torch.float32, torch.bfloat16):
+    if act_dt not in (torch.float32, torch.bfloat16) or split:      # (bf16 -> fp32 is exact)
         students = [s.float() for s in students]
         act_dt = torch.float32
     teachers = [t if t.dtype == act_dt else t.to(act_dt) for t in teachers]
@@ -117,7 +134,7 @@ def _prepare(students: Sequence[torch.Tensor], teachers: Sequence[torch.Tensor],
     proj_t = proj_t.detach().to(device=dev, dtype=torch.float32).contiguous()
     logt = log_temperatures.detach().to(device=dev, dtype=torch.float32).contiguous()
     shape = Shape(B=B, Ns=Ns, Nt=Nt, Ds=Ds, Dt=Dt, Lt=len(teachers), P=len(students), H=H, has_cls=attn_code,
-                  act_dtype=_dtype_code(students[0]), attn_dtype=_dtype_code(attns[0]) if attns else DTYPE_F32, world_size=world_size,
+                  act_dtype=DTYPE_F32_SPLIT if split else _dtype_code(students[0]), attn_dtype=_dtype_code(attns[0]) if attns else DTYPE_F32, world_size=world_size,
                   polar_steps=int(polar_steps), mode=int(mode))
     inp = Inputs()
     for i, s in enumerate(students):
@@ -167,15 +184,17 @@ def _allreduce_sum(dist, t: torch.Tensor):
 # --------------------------------------------------------------------------------------------- custom ops
 @torch.library.custom_op("basd_b200::geo_forward", mutates_args=())
 def geo_forward(students: List[torch.Tensor], teachers: List[torch.Tensor], attns: List[torch.Tensor], proj_s: torch.Tensor,
-                proj_t: torch.Tensor, log_temperatures: torch.Tensor, has_cls: bool, polar_steps: int, mode: int) -> List[torch.Tensor]:
-    """(polar_steps / mode have no defaults on purpose: torch drops default-valued arguments from the autograd inputs.)
+                proj_t: torch.Tensor, log_temperatures: torch.Tensor, has_cls: bool, polar_steps: int, mode: int,
+                token_precision: str) -> List[torch.Tensor]:
+    """(polar_steps / mode / token_precision have no defaults on purpose: torch drops default-valued arguments from the autograd inputs.)
     mode: MODE_LOSS (the geometric term of BASDLoss), MODE_PAIR (geometric_relational_loss of one pair), MODE_SELECTOR
-    (mixing weights only; differentiable through output 3).
+    (mixing weights only; differentiable through output 3).  token_precision: "bf16" or "fp32" (TOKEN_PRECISIONS).
     Returns [geo_loss (0-dim fp32), workspace (uint8), ranks (int32 [Lt]), mixing weights (fp32 [P, Lt]),
     polar residual (fp32 [1]: largest ||X X^T - I||_F going into the last Newton-Schulz step; <= 0.1 = converged)]."""
     lib = _lib.load()
     dist, world = _world()
-    shape, inp, keep = _prepare(students, teachers, attns, proj_s, proj_t, log_temperatures, has_cls, world, polar_steps, mode)
+    shape, inp, keep = _prepare(students, teachers, attns, proj_s, proj_t, log_temperatures, has_cls, world, polar_steps, mode,
+                                token_precision)
     nbytes = ctypes.c_size_t()
     _lib.check(lib.basd_workspace_bytes(ctypes.byref(shape), ctypes.byref(nbytes)), "basd_workspace_bytes")
     dev = students[0].device
@@ -196,23 +215,23 @@ def geo_forward(students: List[torch.Tensor], teachers: List[torch.Tensor], attn
     return [geo, ws, ranks, w, resid]
 
 
-def _fake_workspace_bytes(students, teachers, attns, has_cls, mode=MODE_LOSS) -> int:
+def _fake_workspace_bytes(students, teachers, attns, has_cls, mode=MODE_LOSS, token_precision="bf16") -> int:
     """Same size as the real op's workspace (basd_workspace_bytes is host-only arithmetic on the shape)."""
     B, Ns, Ds = students[0].shape
     _, Nt, Dt = teachers[0].shape
     code = lambda t: DTYPE_BF16 if t.dtype == torch.bfloat16 else DTYPE_F32
     shape = Shape(B=B, Ns=Ns, Nt=Nt, Ds=Ds, Dt=Dt, Lt=len(teachers), P=len(students), H=attns[0].shape[1] if attns else 1, has_cls=int(has_cls),
-                  act_dtype=code(students[0]), attn_dtype=code(attns[0]) if attns else DTYPE_F32, world_size=_world()[1], mode=int(mode))
+                  act_dtype=DTYPE_F32_SPLIT if _split_tokens(students, teachers, token_precision) else code(students[0]), attn_dtype=code(attns[0]) if attns else DTYPE_F32, world_size=_world()[1], mode=int(mode))
     nbytes = ctypes.c_size_t()
     _lib.check(_lib.load().basd_workspace_bytes(ctypes.byref(shape), ctypes.byref(nbytes)), "basd_workspace_bytes")
     return int(nbytes.value)
 
 
 @geo_forward.register_fake
-def _(students, teachers, attns, proj_s, proj_t, log_temperatures, has_cls, polar_steps, mode):
+def _(students, teachers, attns, proj_s, proj_t, log_temperatures, has_cls, polar_steps, mode, token_precision):
     dev = students[0].device
     return [torch.empty((), dtype=torch.float32, device=dev),
-            torch.empty(_fake_workspace_bytes(students, teachers, attns, has_cls, mode), dtype=torch.uint8, device=dev),
+            torch.empty(_fake_workspace_bytes(students, teachers, attns, has_cls, mode, token_precision), dtype=torch.uint8, device=dev),
             torch.empty(len(teachers), dtype=torch.int32, device=dev),
             torch.empty(len(students), len(teachers), dtype=torch.float32, device=dev),
             torch.empty(1, dtype=torch.float32, device=dev)]
@@ -221,12 +240,12 @@ def _(students, teachers, attns, proj_s, proj_t, log_temperatures, has_cls, pola
 @torch.library.custom_op("basd_b200::geo_backward", mutates_args=("workspace",))
 def geo_backward(grad_geo: torch.Tensor, workspace: torch.Tensor, students: List[torch.Tensor], teachers: List[torch.Tensor],
                  attns: List[torch.Tensor], proj_s: torch.Tensor, proj_t: torch.Tensor, log_temperatures: torch.Tensor,
-                 has_cls: bool, mode: int, grad_w: torch.Tensor) -> List[torch.Tensor]:
+                 has_cls: bool, mode: int, grad_w: torch.Tensor, token_precision: str) -> List[torch.Tensor]:
     """Returns [grad_log_temperatures, grad_student_0, ..., grad_student_{P-1}].  grad_w: d(total)/d(mixing weights) [P, Lt]
     in MODE_SELECTOR (then grad_geo is the scalar that multiplies it), an empty tensor otherwise."""
     lib = _lib.load()
     dist, world = _world()
-    shape, inp, keep = _prepare(students, teachers, attns, proj_s, proj_t, log_temperatures, has_cls, world, 0, mode)
+    shape, inp, keep = _prepare(students, teachers, attns, proj_s, proj_t, log_temperatures, has_cls, world, 0, mode, token_precision)
     dev = students[0].device
     with torch.cuda.device(dev):
         st = _stream_ptr(dev)
@@ -250,7 +269,7 @@ def geo_backward(grad_geo: torch.Tensor, workspace: torch.Tensor, students: List
 
 
 @geo_backward.register_fake
-def _(grad_geo, workspace, students, teachers, attns, proj_s, proj_t, log_temperatures, has_cls, mode, grad_w):
+def _(grad_geo, workspace, students, teachers, attns, proj_s, proj_t, log_temperatures, has_cls, mode, grad_w, token_precision):
     return [torch.empty_like(log_temperatures, dtype=torch.float32)] + [torch.empty_like(s) for s in students]
 
 
@@ -259,6 +278,7 @@ def _setup_context(ctx, inputs, output):
     ctx.n_students, ctx.n_teachers, ctx.n_attns = len(students), len(teachers), len(attns)
     ctx.has_cls = has_cls
     ctx.mode = int(inputs[8])
+    ctx.token_precision = inputs[9]
     ctx.student_dtypes = [s.dtype for s in students]
     # only geo_loss carries a gradient; without this autograd materialises zeros_like() for every other output in
     # backward, the multi-GB uint8 workspace included (0.85 ms of fill kernels per step at B=256)
@@ -280,9 +300,9 @@ def _backward(ctx, grads):
         grad_geo = torch.ones((), device=ws.device)
     elif grad_geo is None:
         grad_geo = torch.zeros((), device=ws.device)
-    out = geo_backward(grad_geo, ws, students, teachers, attns, proj_s, proj_t, logt, ctx.has_cls, ctx.mode, grad_w)
+    out = geo_backward(grad_geo, ws, students, teachers, attns, proj_s, proj_t, logt, ctx.has_cls, ctx.mode, grad_w, ctx.token_precision)
     gs = [g.to(dt) if g.dtype != dt else g for g, dt in zip(out[1:], ctx.student_dtypes)]
-    return gs, [None] * Lt, [None] * La, None, None, out[0].to(logt.dtype), None, None, None
+    return gs, [None] * Lt, [None] * La, None, None, out[0].to(logt.dtype), None, None, None, None
 
 
 geo_forward.register_autograd(_backward, setup_context=_setup_context)
@@ -539,11 +559,13 @@ _align_token_count = align_token_count      # the reference's (private) name
 
 
 def geometric_relational_loss(student_tokens: torch.Tensor, teacher_tokens: torch.Tensor, teacher_attn: torch.Tensor, *,
-                              has_cls_token: bool, polar_steps: int = 0) -> torch.Tensor:
+                              has_cls_token: bool, polar_steps: int = 0, token_precision: str = "bf16") -> torch.Tensor:
     """relational.py:5-50 on its own: attention-weighted Procrustes loss of ONE student / teacher pair (teacher tokens already
     on the student's token grid, like combined.py:63-67 hands them over), mean over the batch.  Runs the same kernels as the
     fused loss with the layer selector bypassed (basd_shape.mode = BASD_MODE_PAIR).  The gradient flows to the student tokens;
-    teacher tokens and attention are constants here, as everywhere on this path (teacher.py:123-124,180)."""
+    teacher tokens and attention are constants here, as everywhere on this path (teacher.py:123-124,180).
+    token_precision "fp32": fp32 tokens are carried as split-bf16 pairs instead of being rounded to bf16 (TOKEN_PRECISIONS)."""
+    _check_token_precision(token_precision)
     if student_tokens.device.type != "cuda":
         raise _lib.BasdError("geometric_relational_loss: CUDA tensors required (no CPU fallback)")
     B, n_s, _ = student_tokens.shape
@@ -563,7 +585,7 @@ def geometric_relational_loss(student_tokens: torch.Tensor, teacher_tokens: torc
     dev = student_tokens.device
     none = torch.empty(0, device=dev)
     out = geo_forward([student_tokens], [teacher_tokens.detach()], [teacher_attn.detach()], none, none, torch.zeros(1, device=dev),
-                      bool(has_cls_token), int(polar_steps), MODE_PAIR)
+                      bool(has_cls_token), int(polar_steps), MODE_PAIR, token_precision)
     return out[0]
 
 
@@ -584,6 +606,8 @@ class GrassmannianLayerSelector(nn.Module):
         self.register_buffer("proj_s", proj_s)
         self.register_buffer("proj_t", proj_t)
         self.log_temperatures = nn.Parameter(torch.full((num_extraction_points,), math.log(math.exp(1.0) - 1)))
+        # "bf16" (default): fp32 tokens are rounded to bf16 on entry; "fp32": carried as split-bf16 pairs (TOKEN_PRECISIONS)
+        self.token_precision = "bf16"
 
     @property
     def temperatures(self) -> torch.Tensor:
@@ -601,7 +625,8 @@ class GrassmannianLayerSelector(nn.Module):
         """softmax(-d_Grassmann^2 / tau) of layer_selector.py:86-108 for every (student extraction point, teacher layer):
         [P, Lt] fp32, differentiable w.r.t. the student tokens and log_temperatures (closed-form backward, SURVEY.md B.3-B.5;
         basd_shape.mode = BASD_MODE_SELECTOR).  Updates `subspace_ranks` like layer_selector.py:74."""
-        out = geo_forward(list(students), list(teachers), [], self.proj_s, self.proj_t, self.log_temperatures, True, 0, MODE_SELECTOR)
+        out = geo_forward(list(students), list(teachers), [], self.proj_s, self.proj_t, self.log_temperatures, True, 0, MODE_SELECTOR,
+                          _check_token_precision(self.token_precision))
         self._ranks_dev = out[2]
         self._rank_keys = list(teacher_keys) if teacher_keys is not None else list(range(len(teachers)))
         self.last_mixing_weights = out[3].detach()
@@ -671,6 +696,10 @@ class BASDLoss(nn.Module):
         # looked at by the NEXT forward: above POLAR_RESIDUAL_OK (an ill-conditioned cross-covariance) the step count goes
         # up by one (to at most 16) with a warning - one step late, never a host sync in the step.
         self.polar_steps = 0
+        # How fp32 student / teacher tokens are read: "bf16" (default) rounds them to bf16 on entry, "fp32" carries them as
+        # split-bf16 pairs hi + lo through every kernel (fp32-class accuracy for more bytes and MMAs; DESIGN.md section 8).
+        # bf16 tokens read the same either way.  HostStager follows the module it feeds.
+        self.token_precision = "bf16"
         self.last_polar_residual = None
         self._resid_host = None
         self._resid_event = None
@@ -692,7 +721,8 @@ class BASDLoss(nn.Module):
         self._kt_deficient = ds <= min(ns, nt) - 1 and (nt < ns or dt < ns - 1)
         self._poll_polar_residual()
         geo, _ws, ranks, w, resid = geo_forward(students, teachers, attns, sel.proj_s, sel.proj_t, sel.log_temperatures,
-                                                bool(self.teacher_has_cls_token), int(self.polar_steps), MODE_LOSS)
+                                                bool(self.teacher_has_cls_token), int(self.polar_steps), MODE_LOSS,
+                                                _check_token_precision(self.token_precision))
         sel._ranks_dev, sel._rank_keys = ranks, t_idx
         sel.last_mixing_weights = w
         resid = resid.detach()
@@ -739,6 +769,7 @@ class BASDLoss(nn.Module):
                               "below fp32/split-bf16 resolution; their directions carry unconverged gradient weight", RuntimeWarning)
 
     def forward(self, student_output, targets, student_intermediates, all_teacher_tokens, all_teacher_attns):
+        _check_token_precision(self.token_precision)
         ce_loss = self.base_criterion(student_output, targets)
         geo_loss = self.geo_loss(student_intermediates, all_teacher_tokens, all_teacher_attns)
         self.last_geo_loss, self.last_ce_loss = geo_loss.detach(), ce_loss.detach()
