@@ -175,10 +175,6 @@ int basd_polar_steps(void);
  * kernel (D_s <= 192), 4 otherwise.  For bench.py's launch and byte counts. */
 int basd_polar_launches_per_step(int Ds, int Ns);
 
-/* Development aids (tools/gpu_debug_*.py): phase clocks recorded by one CTA when BASD_POLAR_DBG / BASD_SPECTRAL_DBG is set. */
-int basd_debug_polar_clocks(int which, long long* host_out);
-int basd_debug_spectral_clocks(long long* host_out);
-
 const char* basd_last_error(void);
 const char* basd_version(void);
 

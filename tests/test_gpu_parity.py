@@ -92,7 +92,8 @@ def _stream():
 @pytest.mark.parametrize("variant,M,N,Kd", [(0, 128, 192, 64), (0, 300, 200, 384), (0, 1000, 384, 768),
                                             (1, 192, 192, 1000), (1, 384, 384, 640), (1, 48, 48, 256),
                                             (2, 196, 128, 200), (2, 196, 768, 200), (2, 64, 96, 64),
-                                            (3, 196, 196, 768), (3, 64, 64, 96), (3, 200, 200, 128)])
+                                            (3, 196, 196, 768), (3, 64, 64, 96), (3, 200, 200, 128),
+                                            (3, 9, 9, 64)])
 def test_tcgen05_gemm_variants(lib, cuda_dev, variant, M, N, Kd):
     """Every operand-major combination the path uses (K-major x K-major, MN x MN split-K, K x MN, split-bf16 Gram)
     against an fp32 torch matmul of the same bf16 values: fp32-accumulate accuracy."""

@@ -1,5 +1,5 @@
 """Development aid: determinism and accuracy of the pooled eigen-solver (cluster Jacobi) on repeated launches."""
-import ctypes, os, sys
+import os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 import torch
@@ -26,34 +26,3 @@ for n in (36, 50, 64, 100, 192):
           f"eval err {((outs[0][0].double() - ref).abs().max() / ref.max()).item():.2e}; "
           f"orth {(V @ V.T - torch.eye(n, dtype=torch.float64)).abs().max().item():.2e}")
 
-for n in (48, 96, 192):
-    # time per launch (one problem = one cluster) -> cycles per pair-step
-    torch.manual_seed(n)
-    X = torch.randn(4 * n, n) * (0.97 ** torch.arange(n)); G = (X.T @ X).to(dev)
-    ev = torch.zeros(n, device=dev); evec = torch.zeros(n, n, device=dev); sw = torch.zeros(4, dtype=torch.int32, device=dev)
-    ws = torch.zeros(4 * (2 * n * n + n) + 8192, dtype=torch.uint8, device=dev)
-    for _ in range(3): lib.basd_selftest_eig(G.data_ptr(), n, ev.data_ptr(), evec.data_ptr(), sw.data_ptr(), ws.data_ptr(), st)
-    e0 = torch.cuda.Event(enable_timing=True); e1 = torch.cuda.Event(enable_timing=True)
-    e0.record()
-    for _ in range(20): lib.basd_selftest_eig(G.data_ptr(), n, ev.data_ptr(), evec.data_ptr(), sw.data_ptr(), ws.data_ptr(), st)
-    e1.record(); torch.cuda.synchronize()
-    ms = e0.elapsed_time(e1) / 20
-    steps = sw[0].item() * n // 2
-    print(f"cluster={os.environ.get('BASD_EIG_CLUSTER', 'default')}: {ms*1e3:.0f} us per launch, {sw[0].item()} sweeps, {steps} pair-steps -> {ms*1e-3*1.965e9/steps:.0f} cycles per pair-step (all phases included)")
-    buf = (ctypes.c_longlong * 32)(); lib.basd_debug_spectral_clocks(buf)
-    print("   phase cycles (pre-Jacobi, Jacobi, norms+sort):", list(buf)[:3])
-
-# the angles kernel inside a real step (cfg2, B=64): phase clocks of CTA (0,0)
-import torch.nn as nn
-import bench
-from oracle import synth
-w = bench.workload(64)
-logits, targets, student, teacher, attn = bench.device_inputs(w, dev, 1)
-torch.manual_seed(0)
-m = pkg.BASDLoss(nn.CrossEntropyLoss(), w.Ds, w.Dt, w.student_depth, w.Ns, config=synth.module_config(w), teacher_has_cls_token=True).to(dev)
-for _ in range(2): m.geo_loss(student, teacher, attn)
-torch.cuda.synchronize()
-buf = (ctypes.c_longlong * 32)(); lib.basd_debug_spectral_clocks(buf); c = list(buf)
-names = ["Ur", "W", "-", "jacobi", "distances", "Q", "WQ", "F", "H", "Gamma_sym"]
-print("pooled_eig in the step: pre", c[0], "jacobi", c[1], "post", c[2], "sweeps", c[3])
-print("angles CTA (0,0): k =", c[31], " ".join(f"{n}={c[8+i+1]-c[8+i]}" for i, n in enumerate(names)))

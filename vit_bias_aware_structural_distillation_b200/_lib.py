@@ -40,8 +40,7 @@ EXPORTS = [
     "basd_view", "basd_mp_rank_workspace_bytes", "basd_mp_rank", "basd_selftest_gemm", "basd_selftest_eig",
     "basd_last_error", "basd_version", "basd_timing_enable", "basd_timing_reset", "basd_launch_count", "basd_timing_slots",
     "basd_timing_name", "basd_timing_read", "basd_polar_steps", "basd_polar_launches_per_step", "basd_cls_attention_rows",
-    "basd_copy_cls_rows_h2d", "basd_debug_polar_clocks", "basd_debug_spectral_clocks", "basd_align_tokens", "basd_align_tokens_bwd",
-    "basd_uwso_combine", "basd_query_mean_attention",
+    "basd_copy_cls_rows_h2d", "basd_align_tokens", "basd_align_tokens_bwd", "basd_uwso_combine", "basd_query_mean_attention",
 ]
 
 _lib = None

@@ -83,14 +83,6 @@ extern "C" const char* basd_version(void) { return "basd_b200 0.1 (sm_100a)"; }
 extern "C" int basd_polar_steps(void) { return basd::polar_steps(); }
 namespace basd { int polar_launches_per_step(int Ds, int Ns); }
 extern "C" int basd_polar_launches_per_step(int Ds, int Ns) { return basd::polar_launches_per_step(Ds, Ns); }
-namespace basd { long long* polar_dbg_ptr(int which); }
-// development aid (not in the public header): copies the phase clocks recorded by CTA 0 of one polar GEMM launch
-extern "C" int basd_debug_polar_clocks(int which, long long* host_out) {
-    return cudaMemcpy(host_out, basd::polar_dbg_ptr(which), sizeof(long long) * 128, cudaMemcpyDeviceToHost) == cudaSuccess ? 0 : 1;
-}
-
-namespace basd { int spectral_debug_clocks(long long* host_out); }
-extern "C" int basd_debug_spectral_clocks(long long* host_out) { return basd::spectral_debug_clocks(host_out); }
 
 namespace {
 
@@ -343,23 +335,23 @@ extern "C" int basd_forward_stats(const basd_shape* shape, const basd_inputs* in
     }
     __nv_bfloat16* pt_hi = reinterpret_cast<__nv_bfloat16*>(ws + L.pt_hi);
     __nv_bfloat16* pt_lo = reinterpret_cast<__nv_bfloat16*>(ws + L.pt_lo);
-    Scope* pack_scope = new Scope(1, st, 1 + (packs(s) ? s.Lt + s.P : 0));
-    struct ScopeDel { Scope* p; ~ScopeDel() { delete p; } } pack_del{pack_scope};
-    if (selector) CK(launch_split_bf16(in.proj_t, pt_hi, pt_lo, static_cast<size_t>(s.Ds) * s.Dt, st));
-    if (packs(s)) {
-        // fp32 tokens: rounded to bf16, or (BASD_DTYPE_F32_SPLIT) kept as split pairs, lo halves one block behind the hi halves
-        const bool split = s.act_dtype == BASD_DTYPE_F32_SPLIT;
-        __nv_bfloat16* tpk = reinterpret_cast<__nv_bfloat16*>(ws + L.tpk);
-        __nv_bfloat16* spk = reinterpret_cast<__nv_bfloat16*>(ws + L.spk);
-        const size_t t_block = static_cast<size_t>(s.Lt) * Mt * s.Dt, s_block = static_cast<size_t>(s.P) * Ms * s.Ds;
-        for (int j = 0; j < s.Lt; ++j)
-            CK(launch_pack_bf16(in.teacher[j], 0, in.teacher_strides[0], in.teacher_strides[1], in.teacher_strides[2], s.B, s.Nt, s.Dt,
-                                tpk + static_cast<size_t>(j) * Mt * s.Dt, split ? tpk + t_block + static_cast<size_t>(j) * Mt * s.Dt : nullptr, st));
-        for (int i = 0; i < s.P; ++i)
-            CK(launch_pack_bf16(in.student[i], 0, in.student_strides[0], in.student_strides[1], in.student_strides[2], s.B, s.Ns, s.Ds,
-                                spk + static_cast<size_t>(i) * Ms * s.Ds, split ? spk + s_block + static_cast<size_t>(i) * Ms * s.Ds : nullptr, st));
+    {
+        Scope sc(1, st, 1 + (packs(s) ? s.Lt + s.P : 0));
+        if (selector) CK(launch_split_bf16(in.proj_t, pt_hi, pt_lo, static_cast<size_t>(s.Ds) * s.Dt, st));
+        if (packs(s)) {
+            // fp32 tokens: rounded to bf16, or (BASD_DTYPE_F32_SPLIT) kept as split pairs, lo halves one block behind the hi halves
+            const bool split = s.act_dtype == BASD_DTYPE_F32_SPLIT;
+            __nv_bfloat16* tpk = reinterpret_cast<__nv_bfloat16*>(ws + L.tpk);
+            __nv_bfloat16* spk = reinterpret_cast<__nv_bfloat16*>(ws + L.spk);
+            const size_t t_block = static_cast<size_t>(s.Lt) * Mt * s.Dt, s_block = static_cast<size_t>(s.P) * Ms * s.Ds;
+            for (int j = 0; j < s.Lt; ++j)
+                CK(launch_pack_bf16(in.teacher[j], 0, in.teacher_strides[0], in.teacher_strides[1], in.teacher_strides[2], s.B, s.Nt, s.Dt,
+                                    tpk + static_cast<size_t>(j) * Mt * s.Dt, split ? tpk + t_block + static_cast<size_t>(j) * Mt * s.Dt : nullptr, st));
+            for (int i = 0; i < s.P; ++i)
+                CK(launch_pack_bf16(in.student[i], 0, in.student_strides[0], in.student_strides[1], in.student_strides[2], s.B, s.Ns, s.Ds,
+                                    spk + static_cast<size_t>(i) * Ms * s.Ds, split ? spk + s_block + static_cast<size_t>(i) * Ms * s.Ds : nullptr, st));
+        }
     }
-    delete pack_scope; pack_del.p = nullptr;
     Resolved r;
     if (resolve(s, in, ws, L, &r)) return 1;
     if (!selector) return 0;
@@ -377,21 +369,21 @@ extern "C" int basd_forward_stats(const basd_shape* shape, const basd_inputs* in
     }
     {
         // Grams AND column sums in one pass over the operands (the ones-operand MMA of umma_gemm.cuh): Ds % 4 == 0 is implied by Ds % 8
-        Scope* sc = new Scope(3, st, 6);
-        struct ScDel { Scope*& p; ~ScDel() { delete p; } } sc_del{sc};
         float* gram_part = reinterpret_cast<float*>(ws + L.gram_part);
         const bool fused = gemm_gram_colsum_fused(s.Ds, true);
-        CK(gemm_gram_batched(z, zlo, Mt_rows, s.Ds, s.Lt, stats, static_cast<long long>(stat_stride), gram_part, st, fused));
-        if (r.student_lo[0]) {                  // split-bf16 students (packed: one [P][Ms][Ds] block per half): three-term Grams
-            CK(gemm_gram_batched(r.student[0], r.student_lo[0], Ms, s.Ds, s.P, stats + s.Lt * stat_stride, static_cast<long long>(stat_stride),
-                                 gram_part, st, fused));
-        } else {
-            const void* pts[kMaxPoints];
-            for (int i = 0; i < s.P; ++i) pts[i] = r.student[i];
-            CK(gemm_gram_table(pts, s.P, Ms, s.Ds, stats + s.Lt * stat_stride, static_cast<long long>(stat_stride), gram_part,
-                               r.student_gap ? s.Ns : 0, r.student_bs, st, fused));
+        {
+            Scope sc(3, st, 6);
+            CK(gemm_gram_batched(z, zlo, Mt_rows, s.Ds, s.Lt, stats, static_cast<long long>(stat_stride), gram_part, st, fused));
+            if (r.student_lo[0]) {              // split-bf16 students (packed: one [P][Ms][Ds] block per half): three-term Grams
+                CK(gemm_gram_batched(r.student[0], r.student_lo[0], Ms, s.Ds, s.P, stats + s.Lt * stat_stride, static_cast<long long>(stat_stride),
+                                     gram_part, st, fused));
+            } else {
+                const void* pts[kMaxPoints];
+                for (int i = 0; i < s.P; ++i) pts[i] = r.student[i];
+                CK(gemm_gram_table(pts, s.P, Ms, s.Ds, stats + s.Lt * stat_stride, static_cast<long long>(stat_stride), gram_part,
+                                   r.student_gap ? s.Ns : 0, r.student_bs, st, fused));
+            }
         }
-        delete sc; sc = nullptr;
         if (!fused) {                           // D_s > 192 (two-tile Grams): separate column-sum kernels
             const bool one_launch = Mt_rows == Ms && !r.student_gap;
             Scope sc2(4, st, one_launch ? 2 : 4);
@@ -524,8 +516,8 @@ extern "C" int basd_forward_solve(const basd_shape* shape, const basd_inputs* in
     pa.gwt = reinterpret_cast<float*>(ws + L.gwt);
     pa.loss_b = reinterpret_cast<float*>(ws + L.loss_b);
     pa.dbg = reinterpret_cast<float*>(ws + L.dbg);
-    if (vt) CK(launch_polar_procrustes_vt(pa, st, nullptr));
-    else CK(launch_polar_procrustes(pa, st, nullptr));  // timing slots 10 / 16 / 17 are bracketed inside
+    if (vt) CK(launch_polar_procrustes_vt(pa, st));
+    else CK(launch_polar_procrustes(pa, st));  // timing slots 10 / 16 / 17 are bracketed inside
     float* geo_i = reinterpret_cast<float*>(ws + L.geo_i);
     TIMED(11, 1, CK(launch_loss_reduce(pa.loss_b, pa.dbg, s.P, s.B, geo_i, geo_i + s.P, geo_i + s.P + 1, st)));
     CK(cudaMemcpyAsync(geo_loss, geo_i + s.P, sizeof(float), cudaMemcpyDeviceToDevice, st));

@@ -8,7 +8,6 @@
 
 #include "spectral.h"
 #include "polar_gemm.cuh"
-#include <cstdlib>
 
 #include "polar_fused.cuh"
 #include "umma_gemm.cuh"
@@ -160,7 +159,6 @@ static cudaError_t launch(const GemmMaps& maps, const GemmArgs& args, dim3 grid,
 static inline int cdiv(long long a, long long b) { return static_cast<int>((a + b - 1) / b); }
 
 //                      A_MN   B_MN   BN   MT NA NB T  alias  stages
-using CfgProject = GemmCfg<false, false, 192, 2, 1, 2, 2, false, 2>;     // 256-row tiles: the split P_t tile (49 KB per k-block) is re-read half as often
 using CfgStudentGrad = GemmCfg<false, false, 192, 1, 1, 2, 2, false, 1>;   // one stage (65 KB), 256 TMEM columns: two CTAs per SM overlap each other
 using CfgStudentGrad3 = GemmCfg<false, false, 192, 1, 2, 2, 3, false, 1>;  // split-bf16 students: + S_lo Gamma'_hi (one 81 KB stage)
 using CfgGram    = GemmCfg<true,  true,  192, 2, 1, 1, 1, false, 3>;
@@ -173,24 +171,22 @@ using CfgGramAC  = GemmCfg<true,  true,  192, 2, 1, 1, 1, true,  3, true>;
 using CfgGram3AC = GemmCfg<true,  true,  192, 2, 2, 2, 3, true,  3, true>;
 using CfgTheta   = GemmCfg<false, true,  128, 2, 1, 1, 1, false, 4>;      // self test (single operands)
 template <int BN> using CfgTokenGram = GemmCfg<false, false, BN, 2, 2, 2, 3, true, 3>;
-using CfgTokenGramTiled = GemmCfg<false, false, 192, 2, 2, 2, 3, false, 2>;   // N_s > 256: 256 x 192 output tiles, B loaded separately
 using CfgTestTN  = GemmCfg<false, false, 192, 1, 1, 1, 1, false, 4>;
 
-// Z[j] = X[j] P_t^T for all L_t teacher layers in ONE launch (blockIdx.z = layer; the layers are separate tensors, so each
-// has its own tensor map in maps.a_table).  12 launches of 392 CTAs each left the last wave of every launch 65 % empty.
 // fp32 row-major outputs can leave the persistent kernel as TMA stores (epilogue kind 6) when base, row pitch and batch pitch are
-// 16-byte aligned; BASD_F32_EPI_LANES=1 (read once per process) keeps the per-lane stores (A/B measurements)
+// 16-byte aligned; otherwise (e.g. N_s = 50) as per-lane stores (kind 3)
 static bool f32_tma_ok(const float* out, int ld, long long batch_stride) {
-    static const bool off = [] { const char* e = getenv("BASD_F32_EPI_LANES"); return e && atoi(e) != 0; }();
-    return !off && (reinterpret_cast<uintptr_t>(out) & 15) == 0 && ld % 4 == 0 && batch_stride % 4 == 0;
+    return (reinterpret_cast<uintptr_t>(out) & 15) == 0 && ld % 4 == 0 && batch_stride % 4 == 0;
 }
 
+// Z[j] = X[j] P_t^T for all L_t teacher layers in ONE launch (the layers are separate tensors, so each has its own tensor map
+// in maps.a_tab).  12 launches of 392 CTAs each left the last wave of every launch 65 % empty.
 // The projection on the persistent polar_gemm kernel: work item = (layer, 128-row tile, column tile of <= 256 columns), A = the
 // teacher tokens of that layer through the layer's own tensor map (one exact bf16 buffer: two split terms against P_t hi / lo),
 // operand ring and two TMEM accumulators carried across items, Z leaves as a row-major split pair through swizzled staging and
 // TMA stores (ROWMAJOR epilogue; the rows between the samples of a CLS-stripped view are written as zeros).  The one-tile-per-CTA
-// kernel below ran a two-stage ring and per-lane 32-byte row stores with nothing overlapped: 59 k cycles per 256-row tile against
-// 18 k of MMAs (0.48 ms at cfg2).
+// kernel it replaced ran a two-stage ring and per-lane 32-byte row stores with nothing overlapped: 59 k cycles per 256-row tile
+// against 18 k of MMAs (0.48 ms at cfg2).
 // Split-bf16 teachers (Xlo non-null; X[0] = the hi block [n_layers][M][Dt], Xlo the lo block, both packed): the layers are one
 // batched tensor map per half and the third term X_lo P_hi^T joins the two (a_single = 0).
 static cudaError_t project_persistent(const void* const* X, const __nv_bfloat16* Xlo, int n_layers, size_t M, int Dt, const __nv_bfloat16* Phi,
@@ -268,40 +264,17 @@ static cudaError_t project_persistent(const void* const* X, const __nv_bfloat16*
     return cudaSuccess;
 }
 
-// BASD_PROJECT_TILE=1 (read once per process): keep the one-tile-per-CTA kernel (A/B measurements)
-static bool project_use_tile_kernel() { static const bool v = [] { const char* e = getenv("BASD_PROJECT_TILE"); return e && atoi(e) != 0; }(); return v; }
-
 cudaError_t gemm_project(const void* const* X, int n_layers, size_t M, int Dt, const __nv_bfloat16* Phi, const __nv_bfloat16* Plo, int Ds,
                          __nv_bfloat16* Z, __nv_bfloat16* Zlo, int gap_period, int gap_valid, cudaStream_t st, const __nv_bfloat16* Xlo) {
-    const bool persistent_ok = Ds % 8 == 0 && Dt % 8 == 0 && M < (size_t(1) << 31) - 128;
-    if (Xlo) {                              // split-bf16 teachers: the persistent kernel only (the tile kernel has no X_lo term)
-        if (!persistent_ok || gap_period) {
-            snprintf(g_gemm_err, sizeof g_gemm_err, "project: split-bf16 teachers need dense packed layers, Ds, Dt multiples of 8");
-            return cudaErrorInvalidValue;
-        }
-        return project_persistent(X, Xlo, n_layers, M, Dt, Phi, Plo, Ds, Z, Zlo, 0, 0, st);
+    if (M >= (size_t(1) << 31) - 128) {             // the kernel's row indices are ints
+        snprintf(g_gemm_err, sizeof g_gemm_err, "project: %zu teacher rows, at most 2^31 - 129 supported", M);
+        return cudaErrorInvalidValue;
     }
-    if (persistent_ok && !project_use_tile_kernel())
-        return project_persistent(X, nullptr, n_layers, M, Dt, Phi, Plo, Ds, Z, Zlo, gap_period, gap_valid, st);
-    GemmArgs a;
-    memset(&a, 0, sizeof a);
-    a.gap_period = gap_period; a.gap_valid = gap_valid;
-    a.kb_total = cdiv(Dt, GEMM_BK);
-    a.ld_out = Ds; a.rows_valid = static_cast<int>(M); a.cols_valid = Ds; a.alpha = 1.f;
-    a.out_batch_stride = static_cast<long long>(M) * Ds; a.a_table = 1;
-    for (int j0 = 0; j0 < n_layers; j0 += GEMM_MAX_A_TABLE) {
-        const int nl = n_layers - j0 < GEMM_MAX_A_TABLE ? n_layers - j0 : GEMM_MAX_A_TABLE;
-        GemmMaps maps;
-        memset(&maps, 0, sizeof maps);
-        for (int j = 0; j < nl; ++j)
-            if (make_map(&maps.a_table[j], X[j0 + j], Dt, M, 1, Dt, M * Dt, 128)) return cudaErrorInvalidValue;
-        if (make_map(&maps.b[0], Phi, Dt, Ds, 1, Dt, static_cast<uint64_t>(Ds) * Dt, CfgProject::kBN)) return cudaErrorInvalidValue;
-        if (make_map(&maps.b[1], Plo, Dt, Ds, 1, Dt, static_cast<uint64_t>(Ds) * Dt, CfgProject::kBN)) return cudaErrorInvalidValue;
-        a.out = Z + static_cast<size_t>(j0) * M * Ds; a.aux0 = Zlo + static_cast<size_t>(j0) * M * Ds;
-        cudaError_t e = launch<CfgProject, EpiStoreSplit>(maps, a, dim3(cdiv(Ds, CfgProject::kBN), cdiv(M, CfgProject::kMT * 128), nl), st);
-        if (e != cudaSuccess) return e;
+    if (Xlo && gap_period) {                        // split-bf16 teachers arrive packed: dense layers
+        snprintf(g_gemm_err, sizeof g_gemm_err, "project: split-bf16 teachers need dense packed layers");
+        return cudaErrorInvalidValue;
     }
-    return cudaSuccess;
+    return project_persistent(X, Xlo, n_layers, M, Dt, Phi, Plo, Ds, Z, Zlo, gap_period, gap_valid, st);
 }
 
 // out[b][e] = sum over the n_splits slices of part[(b * n_splits + s) * elems + e], s ascending: fixed order
@@ -459,7 +432,7 @@ static cudaError_t token_gram_impl(const __nv_bfloat16* Thi, const __nv_bfloat16
 // K[z] = T[z] T[z]^T on the persistent polar_gemm kernel: T (row-major split pair [Ns][Dt]) is both operands, work item =
 // (sample, 128-row tile, column tile); with one column tile (Ns <= 256) the A tile is read out of the B tile (no A loads; the
 // second row tile of a sample re-reads the B tile from L2), the fp32 result leaves from the epilogue warps while the next item's
-// MMAs fill the other TMEM accumulator.  The one-tile-per-CTA kernel below (both row tiles against one load of T, nothing
+// MMAs fill the other TMEM accumulator.  The one-tile-per-CTA kernel above (both row tiles against one load of T, nothing
 // overlapped) took 69 k cycles per sample against 30 k of MMAs (0.24 ms at cfg2).
 static cudaError_t token_gram_persistent(const __nv_bfloat16* Thi, const __nv_bfloat16* Tlo, int batches, int Ns, int Dt, float* Ktt,
                                          cudaStream_t st) {
@@ -508,29 +481,10 @@ static cudaError_t token_gram_persistent(const __nv_bfloat16* Thi, const __nv_bf
     kern<<<a.n_items < sm_count ? a.n_items : sm_count, PG_THREADS, smem, st>>>(maps, a);
     return cudaGetLastError();
 }
-// BASD_TOKEN_GRAM_TILE=1 (read once per process): keep the one-tile-per-CTA kernels (A/B measurements)
-static bool token_gram_use_tile_kernel() { static const bool v = [] { const char* e = getenv("BASD_TOKEN_GRAM_TILE"); return e && atoi(e) != 0; }(); return v; }
-
 cudaError_t gemm_token_gram(const __nv_bfloat16* Thi, const __nv_bfloat16* Tlo, int batches, int Ns, int Dt, float* Ktt, cudaStream_t st) {
-    if (Dt % 8 == 0 && Ns >= 16 && !token_gram_use_tile_kernel()) return token_gram_persistent(Thi, Tlo, batches, Ns, Dt, Ktt, st);
-    if (Ns <= 64) return token_gram_impl<64>(Thi, Tlo, batches, Ns, Dt, Ktt, st);
-    if (Ns <= 128) return token_gram_impl<128>(Thi, Tlo, batches, Ns, Dt, Ktt, st);
-    if (Ns <= 208) return token_gram_impl<208>(Thi, Tlo, batches, Ns, Dt, Ktt, st);
-    if (Ns <= 256) return token_gram_impl<256>(Thi, Tlo, batches, Ns, Dt, Ktt, st);
-    // more than one output tile per sample (e.g. 576 tokens at 384 px)
-    GemmMaps maps;
-    memset(&maps, 0, sizeof maps);
-    const __nv_bfloat16* tp[2] = {Thi, Tlo};
-    for (int i = 0; i < 2; ++i) {
-        if (make_map(&maps.a[i], tp[i], Dt, Ns, batches, Dt, static_cast<uint64_t>(Ns) * Dt, 128)) return cudaErrorInvalidValue;
-        if (make_map(&maps.b[i], tp[i], Dt, Ns, batches, Dt, static_cast<uint64_t>(Ns) * Dt, CfgTokenGramTiled::kBN)) return cudaErrorInvalidValue;
-    }
-    GemmArgs a;
-    memset(&a, 0, sizeof a);
-    a.kb_total = cdiv(Dt, GEMM_BK);
-    a.a_batched = 1; a.b_batched = 1;
-    a.out = Ktt; a.out_batch_stride = static_cast<long long>(Ns) * Ns; a.ld_out = Ns; a.rows_valid = Ns; a.cols_valid = Ns; a.alpha = 1.f;
-    return launch<CfgTokenGramTiled, EpiStoreF32>(maps, a, dim3(cdiv(Ns, CfgTokenGramTiled::kBN), cdiv(Ns, CfgTokenGramTiled::kMT * 128), batches), st);
+    // fewer than 16 tokens (e.g. a 3 x 3 teacher grid in the token-space form): the one-tile-per-CTA kernel
+    if (Ns < 16) return token_gram_impl<64>(Thi, Tlo, batches, Ns, Dt, Ktt, st);
+    return token_gram_persistent(Thi, Tlo, batches, Ns, Dt, Ktt, st);
 }
 
 // D[z] = Theta[z] (Ns x Ns, row-major split pair, pitch NsPad) * T[z] (Ns x Dt, row-major split pair): the persistent polar_gemm
@@ -805,12 +759,7 @@ cudaError_t polar_fused_abm(const SplitMat& T, const SplitMat& W, const SplitMat
         if (e != cudaSuccess) return e;
         configured[dev] = true;
     }
-    // development knobs, read once per process: BASD_POLAR_FUSED_GRID (CTAs), BASD_POLAR_FUSED_STAGGER (cycles, odd CTAs)
-    static const int knob_grid = [] { const char* e = getenv("BASD_POLAR_FUSED_GRID"); return e ? atoi(e) : 0; }();
-    static const int knob_stagger = [] { const char* e = getenv("BASD_POLAR_FUSED_STAGGER"); return e ? atoi(e) : 0; }();
-    a.stagger = knob_stagger;
-    int sm_count = device_sm_count();
-    if (knob_grid > 0 && knob_grid < sm_count) sm_count = knob_grid;
+    const int sm_count = device_sm_count();
     const int grid = batches < sm_count ? batches : sm_count;
     polar_fused_abm_kernel<<<grid, PF_THREADS, smem, st>>>(maps, a);
     return cudaGetLastError();
@@ -819,7 +768,7 @@ cudaError_t polar_fused_abm(const SplitMat& T, const SplitMat& W, const SplitMat
 // variant 0: C[M][N] = A[M][K] B[N][K]^T          (both K-major)
 // variant 1: C[M][N] = A[K][M]^T B[K][N]          (both MN-major; split-K + atomics; C pre-zeroed)
 // variant 2: C[M][N] = A[M][K] B[K][N]            (A K-major, B MN-major)
-// variant 3: C[M][M] = A A^T + A B^T + B A^T      (token_gram path: A = hi [M][K], B = lo [M][K]; M <= 208)
+// variant 3: C[M][M] = A A^T + A B^T + B A^T      (token_gram path: A = hi [M][K], B = lo [M][K])
 cudaError_t gemm_selftest(int variant, const __nv_bfloat16* A, const __nv_bfloat16* B, float* C, int M, int N, int K,
                           cudaStream_t st) {
     GemmMaps maps;

@@ -13,8 +13,6 @@
 // pushing the top singular value into the divergent region.
 // All products are one-CTA-per-problem tcgen05 GEMMs on split-bf16 operands (polar_gemm.cuh).
 // Requires rank(C) = D_s, i.e. D_s <= N - 1 and a teacher token Gram of rank >= D_s.
-#include <cstdlib>
-
 #include "cta_linalg.cuh"
 #include "polar_gemm.cuh"
 #include "spectral.h"
@@ -24,7 +22,6 @@ namespace basd {
 namespace {
 
 constexpr int kPolarSteps = kPolarStepsDefault;      // rows of the schedule below
-constexpr int kPolarChunk = 0;            // problems per launch of the product chain (0 = all); BASD_POLAR_CHUNK overrides
 // minimax odd quintics on [l_k, 1.03] (l_0 = 3e-5), each rescaled to a maximum of 1: tools/ns_schedule.py 3e-5 10 1.03
 // l_k: 3.0e-5 1.0e-4 4.2e-4 1.7e-3 7.1e-3 2.9e-2 0.118 0.42 0.906 0.99967 -> 0.999996
 const float kPolarCoef[kPolarSteps][3] = {
@@ -48,17 +45,6 @@ __host__ inline const float* polar_coef(int k, int steps) {
     return kPolarCoef[idx < 0 ? 0 : idx];
 }
 
-// ------------------------------------------------------------------------------------------------
-// prep_student: s_w = sqrt(a) (s - mu_s)  ->  SW [N][Ds] (split), W_0 = s_w^T [Ds][Np] (split), ksd, tr_s
-// one CTA per problem; the whole s_w tile lives in shared memory (fp32, padded rows)
-// ------------------------------------------------------------------------------------------------
-__device__ __forceinline__ void store_split2(__nv_bfloat16* hi, __nv_bfloat16* lo, size_t idx, float v0, float v1) {   // idx even
-    const __nv_bfloat16 h0 = __float2bfloat16(v0), h1 = __float2bfloat16(v1);
-    __nv_bfloat162 hv; hv.x = h0; hv.y = h1;
-    *reinterpret_cast<__nv_bfloat162*>(hi + idx) = hv;
-    *reinterpret_cast<__nv_bfloat162*>(lo + idx) = __floats2bfloat162_rn(v0 - __bfloat162float(h0), v1 - __bfloat162float(h1));
-}
-
 // eight consecutive values -> one 16-byte store per half (idx a multiple of 8)
 __device__ __forceinline__ void store_split8(__nv_bfloat16* hi, __nv_bfloat16* lo, size_t idx, const float* v) {
     uint32_t hw[4], lw[4];
@@ -75,78 +61,10 @@ __device__ __forceinline__ void store_split8(__nv_bfloat16* hi, __nv_bfloat16* l
 }
 
 constexpr int kPrepThreads = 512;
-__global__ void __launch_bounds__(kPrepThreads)
-polar_prep_student_kernel(PolarArgs g) {
-    extern __shared__ float sm[];
-    const int N = g.Ns, D = g.Ds, ldS = D + 1;
-    float* sw = sm;                                   // [N][D+1]
-    float* a_s = sw + static_cast<size_t>(N) * ldS;   // [N]
-    float* q_s = a_s + N;
-    float* mu = q_s + N;                              // [D]
-    float* red = mu + D;                              // 40
-    const int prob = blockIdx.x;
-    const int i = prob / g.B, b = prob % g.B;
-    const __nv_bfloat16* S = g.student[i] + static_cast<size_t>(b) * g.student_bs;
-    for (int n = threadIdx.x; n < N; n += blockDim.x) {
-        const float a = g.a[static_cast<size_t>(prob) * N + n];
-        a_s[n] = a;
-        q_s[n] = sqrtf(a);
-    }
-    // raw tokens -> shared memory (bf16x2 loads, D is even)
-    for (int t = threadIdx.x; t < N * D / 2; t += blockDim.x) {
-        const float2 v = __bfloat1622float2(reinterpret_cast<const __nv_bfloat162*>(S)[t]);
-        const int n = (2 * t) / D, d = (2 * t) % D;
-        sw[n * ldS + d] = v.x;
-        sw[n * ldS + d + 1] = v.y;
-    }
-    __syncthreads();
-    for (int d = threadIdx.x; d < D; d += blockDim.x) {
-        float m = 0.f;
-        for (int n = 0; n < N; ++n) m = fmaf(a_s[n], sw[n * ldS + d], m);
-        mu[d] = m;
-    }
-    __syncthreads();
-    for (int t = threadIdx.x; t < N * D; t += blockDim.x) {
-        const int n = t / D, d = t % D;
-        sw[n * ldS + d] = q_s[n] * (sw[n * ldS + d] - mu[d]);
-    }
-    __syncthreads();
-    float* ksd = g.vec + static_cast<size_t>(prob) * 4 * N;
-    float part = 0.f;
-    {
-        const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nw = blockDim.x >> 5;
-        for (int n = warp; n < N; n += nw) {
-            float s = 0.f;
-            for (int d = lane; d < D; d += 32) { const float v = sw[n * ldS + d]; s = fmaf(v, v, s); }
-            s = warp_sum(s);
-            if (lane == 0) { ksd[n] = s; part += s; }
-        }
-    }
-    const float tr_s = cta_sum(part, red);
-    if (threadIdx.x == 0) g.scal[prob * 4 + 1] = tr_s;
-    // SW = s_w  [N][Ds], tiled [d block][n][64]: pairs of consecutive d
-    __nv_bfloat16* swh = g.SW.hi + prob * g.SW.batch_stride;
-    __nv_bfloat16* swl = g.SW.lo + prob * g.SW.batch_stride;
-    const int Dp = (D + 63) / 64 * 64;
-    for (int t = threadIdx.x; t < N * Dp / 2; t += blockDim.x) {
-        const int e = 2 * t;                                  // storage index: ((cb * N + n) * 64 + j)
-        const int j = e % 64, n = (e / 64) % N, d = (e / (64 * N)) * 64 + j;
-        store_split2(swh, swl, e, d < D ? sw[n * ldS + d] : 0.f, d + 1 < D ? sw[n * ldS + d + 1] : 0.f);
-    }
-    if (g.vt) return;
-    // W_0 = s_w^T [Ds][N], tiled [n block][d][64]: pairs of consecutive n; padding columns stored as zeros
-    __nv_bfloat16* wh = g.W.hi + prob * g.W.batch_stride;
-    __nv_bfloat16* wl = g.W.lo + prob * g.W.batch_stride;
-    const int Np = (N + 63) / 64 * 64;
-    for (int t = threadIdx.x; t < D * Np / 2; t += blockDim.x) {
-        const int e = 2 * t;                                  // storage index: ((nb * D + d) * 64 + j)
-        const int j = e % 64, d = (e / 64) % D, n = (e / (64 * D)) * 64 + j;
-        store_split2(wh, wl, e, n < N ? sw[n * ldS + d] : 0.f, n + 1 < N ? sw[(n + 1) * ldS + d] : 0.f);
-    }
-}
 
 // ------------------------------------------------------------------------------------------------
-// prep_student, D_s a multiple of 8: the raw bf16 tile stays in shared memory as it was read (16-byte loads, 78 KB
+// prep_student: s_w = sqrt(a) (s - mu_s)  ->  SW [N][Ds] (split), W_0 = s_w^T [Ds][Np] (split), ksd, tr_s; one CTA per problem.
+// D_s is a multiple of 8 (check_shape): the raw bf16 tile stays in shared memory as it was read (16-byte loads, 78 KB
 // instead of 151 KB of fp32 -> two CTAs per SM overlap each other's load / compute / store phases) and
 // s_w = sqrt(a) (s - mu) is recomputed where it is consumed; every global access is 16 bytes wide.
 // ------------------------------------------------------------------------------------------------
@@ -736,27 +654,11 @@ int polar_fro_slots(int core) {
     const int t = (core + 127) / 128;
     return (4 * t * t + 7) & ~7;
 }
-// Development knobs, read ONCE per process (C++11 thread-safe static initialisation), never on the launch path:
-//   BASD_POLAR_FUSED=0  keep G2 and G3 as two launches      BASD_POLAR_CHUNK=n  problems per launch chain
-//   BASD_POLAR_DBG=1    record the phase clocks of one launch per product (tools/gpu_debug_clocks.py)
-struct PolarKnobs {
-    int fused, chunk, dbg;
-    PolarKnobs() {
-        const char* e = getenv("BASD_POLAR_FUSED"); fused = e ? atoi(e) : 1;
-        e = getenv("BASD_POLAR_CHUNK"); chunk = e ? atoi(e) : kPolarChunk;
-        dbg = getenv("BASD_POLAR_DBG") ? 1 : 0;
-    }
-};
-static const PolarKnobs& polar_knobs() { static const PolarKnobs k; return k; }
-static bool polar_use_fused(int D, int N) { return polar_knobs().fused != 0 && polar_fused_supported(D, N); }
-int polar_launches_per_step(int Ds, int Ns) { return polar_use_fused(Ds, Ns) ? 3 : 4; }
-
-__device__ long long g_polar_dbg[4][16 * 8];
-long long* polar_dbg_ptr(int which) { long long* p = nullptr; cudaGetSymbolAddress(reinterpret_cast<void**>(&p), g_polar_dbg); return p + which * 128; }
+int polar_launches_per_step(int Ds, int Ns) { return polar_fused_supported(Ds, Ns) ? 3 : 4; }
 
 #define PCK(expr) do { cudaError_t _e = (expr); if (_e != cudaSuccess) return _e; } while (0)
 
-// prep_student for D_s % 8 == 0 (both polar forms): the raw token tile is staged in shared memory when it fits (split-bf16
+// prep_student (both polar forms): the raw token tile is staged in shared memory when it fits (split-bf16
 // students stage their lo tile too), otherwise read from global memory
 template <bool SPLIT>
 static cudaError_t launch_prep_student_vec(const PolarArgs& g, cudaStream_t st) {
@@ -777,214 +679,174 @@ static cudaError_t launch_prep_student_vec(const PolarArgs& g, cudaStream_t st) 
     return g.student_lo[0] ? launch_prep_student_vec<true>(g, st) : launch_prep_student_vec<false>(g, st);
 }
 
-cudaError_t launch_polar_procrustes(const PolarArgs& g, cudaStream_t st, int* launches) {
+cudaError_t launch_polar_procrustes(const PolarArgs& g, cudaStream_t st) {
     const int N = g.Ns, D = g.Ds, nprob = g.n_problems;
-    int count = 0;
     {
         TimingScope ts(kSlotPolarPrep, st, 2);
-        if (D % 8 == 0) {
-            PCK(launch_prep_student_vec(g, st));
-        } else {
-            if (g.student_lo[0]) return cudaErrorInvalidValue;      // (check_shape requires D_s % 8 == 0)
-            const size_t smem = (static_cast<size_t>(N) * (D + 1) + 2 * N + D + 64) * sizeof(float);
-            PCK(cudaFuncSetAttribute(polar_prep_student_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
-            polar_prep_student_kernel<<<nprob, kPrepThreads, smem, st>>>(g);
-        }
-        PCK(cudaGetLastError());
+        PCK(launch_prep_student_vec(g, st));
         polar_prep_teacher_kernel<<<nprob, 256, (3 * N + 64) * sizeof(float), st>>>(g);
         PCK(cudaGetLastError());
-        count += 2;
     }
-    float* fro2_dense = g.fro2;                // partial traces of the first A = T W^T per problem (their sum = ||C||_F^2)
-    PCK(cudaMemsetAsync(fro2_dense, 0, sizeof(float) * nprob * g.fro_slots, st));
+    // partial traces of the first A = T W^T per problem (their sum = ||C||_F^2)
+    PCK(cudaMemsetAsync(g.fro2, 0, sizeof(float) * nprob * g.fro_slots, st));
 
-    // The chain of products is sequentially dependent per problem but every launch batches many problems.  Problems are
-    // walked in chunks small enough for a chunk's matrices (~0.8 MB live per problem) to stay in the 126 MB L2 from one
-    // launch to the next; one chunk = one full Newton-Schulz run.  chunk = 0: all problems per launch (HBM streaming).
-    const int chunk_cfg = polar_knobs().chunk;
-    const bool dbg_clocks = polar_knobs().dbg != 0;
-    const int chunk = (chunk_cfg <= 0 || chunk_cfg > nprob) ? nprob : chunk_cfg;
-    const int n_chunks = (nprob + chunk - 1) / chunk;
-    const bool fused = polar_use_fused(D, N);
-    auto at = [](const SplitMat& m, int z0) { SplitMat r = m; r.hi += z0 * m.batch_stride; r.lo += z0 * m.batch_stride; return r; };
+    // The chain of products is sequentially dependent per problem; every launch batches all problems.
+    const bool fused = polar_fused_supported(D, N);
     const int steps = g.steps >= kPolarStepsMin && g.steps <= kPolarStepsMax ? g.steps : kPolarSteps;
     PCK(cudaMemsetAsync(g.resid, 0, sizeof(float) * nprob * g.fro_slots, st));
-    TimingScope* gemm_scope = new TimingScope(kSlotPolarGemm, st, n_chunks * ((fused ? 3 : 4) * steps + 2));
-    struct Del { TimingScope*& p; ~Del() { delete p; } } gemm_del{gemm_scope};
-    for (int z0 = 0; z0 < nprob; z0 += chunk) {
-        const int nz = nprob - z0 < chunk ? nprob - z0 : chunk;
+    {
+        TimingScope ts(kSlotPolarGemm, st, (fused ? 3 : 4) * steps + 2);
         // Step 0 runs on the unnormalised W_0 = s_w^T; r = 1 / ||C||_F^2 (trace of W_0 K_t W_0^T, accumulated by the first
         // A product) enters the later epilogues of that step as a per-problem scalar.
-        SplitMat Wc = at(g.W, z0), Wn = at(g.W2, z0);
-        const SplitMat T = at(g.T, z0), A = at(g.A, z0), Bm = at(g.Bm, z0), Kt = at(g.Kt, z0), SW = at(g.SW, z0);
-        float* fro2 = fro2_dense + static_cast<size_t>(z0) * g.fro_slots;
+        SplitMat Wc = g.W, Wn = g.W2;
+        const SplitMat &T = g.T, &A = g.A, &Bm = g.Bm, &Kt = g.Kt;
         int dir = 0;                           // alternate the problem order launch by launch (L2 reuse of the previous output)
-        float* resid = g.resid + static_cast<size_t>(z0) * g.fro_slots;
         for (int k = 0; k < steps; ++k) {
             const float* coef = polar_coef(k, steps);
             const float ca = coef[0], cb = coef[1], cc = coef[2];
             const bool first = k == 0, last = k == steps - 1;
-            const float* norm = first ? fro2 : nullptr;
+            const float* norm = first ? g.fro2 : nullptr;
             PolarGemmArgs a;
             // G1: T = W K_t
             memset(&a, 0, sizeof a);
             a.epi = PG_EPI_SPLIT; a.out_hi = T.hi; a.out_lo = T.lo; a.out_stride = T.batch_stride; a.scale_c = 1.f;
-            if (k == 3 && z0 == 0 && dbg_clocks) a.dbg_clock = polar_dbg_ptr(0);
             a.reverse = (dir++) & 1;
-            PCK(polar_gemm(false, Wc, Kt, nz, a, st));
+            PCK(polar_gemm(false, Wc, Kt, nprob, a, st));
             if (fused) {
                 // G2 + G3 in one kernel: A = T W^T stays in TMEM / shared memory, Bm = a I + b (rA) + c (rA)^2 leaves
                 // (step 0: trace(A) = ||C||_F^2 is reduced inside and written to fro2 for G4's epilogue)
                 PolarFusedArgs f;
                 memset(&f, 0, sizeof f);
-                f.ca = ca; f.cb = cb; f.cc = cc; f.first = first ? 1 : 0; f.fro2 = fro2; f.fro_slots = g.fro_slots;
-                f.resid = last ? resid : nullptr;
-                if (k == 3 && z0 == 0 && dbg_clocks) f.dbg_clock = polar_dbg_ptr(1);
+                f.ca = ca; f.cb = cb; f.cc = cc; f.first = first ? 1 : 0; f.fro2 = g.fro2; f.fro_slots = g.fro_slots;
+                f.resid = last ? g.resid : nullptr;
                 f.reverse = (dir++) & 1;
-                PCK(polar_fused_abm(T, Wc, Bm, nz, f, st));
-                count -= 1;
+                PCK(polar_fused_abm(T, Wc, Bm, nprob, f, st));
             } else {
                 // G2: A = T W^T                (step 0: trace(A) = ||C||_F^2, read by the epilogues of G3 / G4 of that step)
                 memset(&a, 0, sizeof a);
                 a.epi = PG_EPI_SPLIT; a.out_hi = A.hi; a.out_lo = A.lo; a.out_stride = A.batch_stride; a.scale_c = 1.f;
-                if (first) { a.trace = fro2; a.fro_slots = g.fro_slots; }
-                if (k == 3 && z0 == 0 && dbg_clocks) a.dbg_clock = polar_dbg_ptr(1);
+                if (first) { a.trace = g.fro2; a.fro_slots = g.fro_slots; }
                 a.reverse = (dir++) & 1;
-                PCK(polar_gemm(false, T, Wc, nz, a, st));
+                PCK(polar_gemm(false, T, Wc, nprob, a, st));
                 // G3: Bm = a I + b (rA) + c (rA)^2   (A is both operands: the A tile aliases the B tile; the b A term is added from
                 //     a TMA-loaded copy of the output-shaped tile of A in the epilogue)
                 memset(&a, 0, sizeof a);
                 a.epi = PG_EPI_SPLIT; a.out_hi = Bm.hi; a.out_lo = Bm.lo; a.out_stride = Bm.batch_stride;
                 a.a_alias_b = 1; a.aux_mode = 1; a.aux_hi = A.hi; a.aux_lo = A.lo;
                 a.aux_c = cb; a.aux_p = first ? 1.f : 0.f; a.scale_c = cc; a.scale_p = first ? 2.f : 0.f; a.diag_add = ca; a.norm2 = norm; a.fro_slots = g.fro_slots;
-                a.resid = last ? resid : nullptr;
-                if (k == 3 && z0 == 0 && dbg_clocks) a.dbg_clock = polar_dbg_ptr(2);
+                a.resid = last ? g.resid : nullptr;
                 a.reverse = (dir++) & 1;
-                PCK(polar_gemm(false, A, A, nz, a, st));
+                PCK(polar_gemm(false, A, A, nprob, a, st));
             }
             // G4: W_next = sqrt(r) Bm W      (W enters as the MN-major B operand; ping-pong buffers)
             memset(&a, 0, sizeof a);
             a.epi = PG_EPI_SPLIT; a.out_hi = Wn.hi; a.out_lo = Wn.lo; a.out_stride = Wn.batch_stride;
             a.scale_c = 1.f; a.scale_p = first ? 0.5f : 0.f; a.norm2 = norm; a.fro_slots = g.fro_slots;
-            if (k == 3 && z0 == 0 && dbg_clocks) a.dbg_clock = polar_dbg_ptr(3);
             a.reverse = (dir++) & 1;
-            PCK(polar_gemm(true, Bm, Wc, nz, a, st));
+            PCK(polar_gemm(true, Bm, Wc, nprob, a, st));
             const SplitMat tmp = Wc; Wc = Wn; Wn = tmp;
-            count += 4;
         }
         PolarGemmArgs a;
         // Gsw = K_t W^T  [N][Ds]
         memset(&a, 0, sizeof a);
-        a.epi = PG_EPI_F32; a.out_f32 = g.Gsw + static_cast<size_t>(z0) * N * D; a.out_f32_stride = static_cast<long long>(N) * D; a.ld_f32 = D;
+        a.epi = PG_EPI_F32; a.out_f32 = g.Gsw; a.out_f32_stride = static_cast<long long>(N) * D; a.ld_f32 = D;
         a.reverse = (dir++) & 1;
-        PCK(polar_gemm(false, Kt, Wc, nz, a, st));
+        PCK(polar_gemm(false, Kt, Wc, nprob, a, st));
         // Psi = s_w W  [N][N]  -> Theta' = 2 (diag(a) - q Psi q - a a^T), stored as a split pair
         memset(&a, 0, sizeof a);
-        a.epi = PG_EPI_THETA; a.out_hi = g.theta + static_cast<size_t>(z0) * N * g.NsPad; a.out_lo = g.theta_lo + static_cast<size_t>(z0) * N * g.NsPad;
+        a.epi = PG_EPI_THETA; a.out_hi = g.theta; a.out_lo = g.theta_lo;
         a.out_stride = static_cast<long long>(N) * g.NsPad; a.ld_out = g.NsPad;
-        a.vec_a = g.a + static_cast<size_t>(z0) * N;
+        a.vec_a = g.a;
         a.reverse = (dir++) & 1;
-        PCK(polar_gemm(true, SW, Wc, nz, a, st));
-        count += 2;
+        PCK(polar_gemm(true, g.SW, Wc, nprob, a, st));
     }
     {
-        delete gemm_scope; gemm_scope = nullptr;
-        TimingScope tf(kSlotPolarFinish, st, 1);
+        TimingScope ts(kSlotPolarFinish, st, 1);
         polar_finish_kernel<<<nprob, 256, (2 * N + 64) * sizeof(float), st>>>(g);
         PCK(cudaGetLastError());
-        count += 1;
     }
-    if (launches) *launches = count;
     return cudaSuccess;
 }
 
-cudaError_t launch_polar_procrustes_vt(const PolarArgs& g, cudaStream_t st, int* launches) {
+cudaError_t launch_polar_procrustes_vt(const PolarArgs& g, cudaStream_t st) {
     const int N = g.Ns, M = g.Nt, D = g.Ds, nprob = g.n_problems;
     if (M > kVtMaxTokens || M > kVtThreads) return cudaErrorInvalidValue;
-    int count = 0;
     {
         TimingScope ts(kSlotPolarPrep, st, 3);
-        if (D % 8 != 0) return cudaErrorInvalidValue;
         PCK(launch_prep_student_vec(g, st));
         const int ld = (M + 3) & ~3;
         const size_t smem_t = (static_cast<size_t>(ld) * M + 2 * N + 3 * M + 64) * sizeof(float);
         PCK(cudaFuncSetAttribute(vt_prep_teacher_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem_t)));
         vt_prep_teacher_kernel<<<nprob, kVtThreads, smem_t, st>>>(g);
         PCK(cudaGetLastError());
-        count += 2;
     }
     const int steps = g.steps >= kPolarStepsMin && g.steps <= kPolarStepsMax ? g.steps : kPolarSteps;
     PCK(cudaMemsetAsync(g.fro2, 0, sizeof(float) * nprob * g.fro_slots, st));
     PCK(cudaMemsetAsync(g.resid, 0, sizeof(float) * nprob * g.fro_slots, st));
-    TimingScope* gemm_scope = new TimingScope(kSlotPolarGemm, st, 3 * steps + 7);
-    struct Del { TimingScope*& p; ~Del() { delete p; } } gemm_del{gemm_scope};
-    PolarGemmArgs a;
-    // X_0 = (F G)^T s_w   [Nt][Ds]  (s_w enters as the MN-major operand), then the augmentation column
-    memset(&a, 0, sizeof a);
-    a.epi = PG_EPI_SPLIT; a.out_hi = g.X0.hi; a.out_lo = g.X0.lo; a.out_stride = g.X0.batch_stride; a.scale_c = 1.f;
-    PCK(polar_gemm(true, g.FGt, g.SW, nprob, a, st));
-    vt_augment_kernel<<<nprob, 256, 0, st>>>(g);
-    PCK(cudaGetLastError());
-    count += 2;
-    SplitMat Xc = g.X0, Xn = g.X1;
-    int dir = 0;
-    for (int k = 0; k < steps; ++k) {
-        const float* coef = polar_coef(k, steps);
-        const float ca = coef[0], cb = coef[1], cc = coef[2];
-        const bool first = k == 0, last = k == steps - 1;
-        const float* norm = first ? g.fro2 : nullptr;
-        // A = X X^T   (step 0: trace(A) = ||X_0^+||_F^2)
-        memset(&a, 0, sizeof a);
-        a.epi = PG_EPI_SPLIT; a.out_hi = g.A.hi; a.out_lo = g.A.lo; a.out_stride = g.A.batch_stride; a.scale_c = 1.f;
-        a.a_alias_b = 1;
-        if (first) { a.trace = g.fro2; a.fro_slots = g.fro_slots; }
-        a.reverse = (dir++) & 1;
-        PCK(polar_gemm(false, Xc, Xc, nprob, a, st));
-        // Bm = a I + b (rA) + c (rA)^2
-        memset(&a, 0, sizeof a);
-        a.epi = PG_EPI_SPLIT; a.out_hi = g.Bm.hi; a.out_lo = g.Bm.lo; a.out_stride = g.Bm.batch_stride;
-        a.a_alias_b = 1; a.aux_mode = 1; a.aux_hi = g.A.hi; a.aux_lo = g.A.lo;
-        a.aux_c = cb; a.aux_p = first ? 1.f : 0.f; a.scale_c = cc; a.scale_p = first ? 2.f : 0.f; a.diag_add = ca; a.norm2 = norm; a.fro_slots = g.fro_slots;
-        a.resid = last ? g.resid : nullptr;
-        a.reverse = (dir++) & 1;
-        PCK(polar_gemm(false, g.A, g.A, nprob, a, st));
-        // X_next = sqrt(r) Bm X
-        memset(&a, 0, sizeof a);
-        a.epi = PG_EPI_SPLIT; a.out_hi = Xn.hi; a.out_lo = Xn.lo; a.out_stride = Xn.batch_stride;
-        a.scale_c = 1.f; a.scale_p = first ? 0.5f : 0.f; a.norm2 = norm; a.fro_slots = g.fro_slots;
-        a.reverse = (dir++) & 1;
-        PCK(polar_gemm(true, g.Bm, Xc, nprob, a, st));
-        Xc = Xn;
-        Xn = (Xc.hi == g.X1.hi) ? g.X2 : g.X1;
-        count += 3;
-    }
-    const int d16 = (D + 15) & ~15;
-    // Gsw = F G X_inf[:, :Ds] = d nuc / d s_w   [Ns][Ds]
-    memset(&a, 0, sizeof a);
-    a.epi = PG_EPI_F32; a.out_f32 = g.Gsw; a.out_f32_stride = static_cast<long long>(N) * D; a.ld_f32 = D; a.n_override = D;
-    PCK(polar_gemm(true, g.FG, Xc, nprob, a, st));
-    // H = X_0 X_inf^T over the student features (the augmentation column left out)
-    memset(&a, 0, sizeof a);
-    a.epi = PG_EPI_SPLIT; a.out_hi = g.Hm.hi; a.out_lo = g.Hm.lo; a.out_stride = g.Hm.batch_stride; a.scale_c = 1.f; a.k_override = d16;
-    PCK(polar_gemm(false, g.X0, Xc, nprob, a, st));
-    // M2 = H G^-1 (I - 1 1^T / Nt),  Theta_raw = G^-T M2
-    memset(&a, 0, sizeof a);
-    a.epi = PG_EPI_SPLIT; a.out_hi = g.M2.hi; a.out_lo = g.M2.lo; a.out_stride = g.M2.batch_stride; a.scale_c = 1.f;
-    PCK(polar_gemm(true, g.Hm, g.GinvC, nprob, a, st));
-    memset(&a, 0, sizeof a);
-    a.epi = PG_EPI_F32; a.out_f32 = g.thraw; a.out_f32_stride = static_cast<long long>(M) * M; a.ld_f32 = M;
-    PCK(polar_gemm(true, g.GinvT, g.M2, nprob, a, st));
-    vt_theta_kernel<<<dim3((M * M + 255) / 256 < 8 ? (M * M + 255) / 256 : 8, nprob), 256, 0, st>>>(g);
-    PCK(cudaGetLastError());
-    count += 5;
     {
-        delete gemm_scope; gemm_scope = nullptr;
-        TimingScope tf(kSlotPolarFinish, st, 1);
+        TimingScope ts(kSlotPolarGemm, st, 3 * steps + 7);
+        PolarGemmArgs a;
+        // X_0 = (F G)^T s_w   [Nt][Ds]  (s_w enters as the MN-major operand), then the augmentation column
+        memset(&a, 0, sizeof a);
+        a.epi = PG_EPI_SPLIT; a.out_hi = g.X0.hi; a.out_lo = g.X0.lo; a.out_stride = g.X0.batch_stride; a.scale_c = 1.f;
+        PCK(polar_gemm(true, g.FGt, g.SW, nprob, a, st));
+        vt_augment_kernel<<<nprob, 256, 0, st>>>(g);
+        PCK(cudaGetLastError());
+        SplitMat Xc = g.X0, Xn = g.X1;
+        int dir = 0;
+        for (int k = 0; k < steps; ++k) {
+            const float* coef = polar_coef(k, steps);
+            const float ca = coef[0], cb = coef[1], cc = coef[2];
+            const bool first = k == 0, last = k == steps - 1;
+            const float* norm = first ? g.fro2 : nullptr;
+            // A = X X^T   (step 0: trace(A) = ||X_0^+||_F^2)
+            memset(&a, 0, sizeof a);
+            a.epi = PG_EPI_SPLIT; a.out_hi = g.A.hi; a.out_lo = g.A.lo; a.out_stride = g.A.batch_stride; a.scale_c = 1.f;
+            a.a_alias_b = 1;
+            if (first) { a.trace = g.fro2; a.fro_slots = g.fro_slots; }
+            a.reverse = (dir++) & 1;
+            PCK(polar_gemm(false, Xc, Xc, nprob, a, st));
+            // Bm = a I + b (rA) + c (rA)^2
+            memset(&a, 0, sizeof a);
+            a.epi = PG_EPI_SPLIT; a.out_hi = g.Bm.hi; a.out_lo = g.Bm.lo; a.out_stride = g.Bm.batch_stride;
+            a.a_alias_b = 1; a.aux_mode = 1; a.aux_hi = g.A.hi; a.aux_lo = g.A.lo;
+            a.aux_c = cb; a.aux_p = first ? 1.f : 0.f; a.scale_c = cc; a.scale_p = first ? 2.f : 0.f; a.diag_add = ca; a.norm2 = norm; a.fro_slots = g.fro_slots;
+            a.resid = last ? g.resid : nullptr;
+            a.reverse = (dir++) & 1;
+            PCK(polar_gemm(false, g.A, g.A, nprob, a, st));
+            // X_next = sqrt(r) Bm X
+            memset(&a, 0, sizeof a);
+            a.epi = PG_EPI_SPLIT; a.out_hi = Xn.hi; a.out_lo = Xn.lo; a.out_stride = Xn.batch_stride;
+            a.scale_c = 1.f; a.scale_p = first ? 0.5f : 0.f; a.norm2 = norm; a.fro_slots = g.fro_slots;
+            a.reverse = (dir++) & 1;
+            PCK(polar_gemm(true, g.Bm, Xc, nprob, a, st));
+            Xc = Xn;
+            Xn = (Xc.hi == g.X1.hi) ? g.X2 : g.X1;
+        }
+        const int d16 = (D + 15) & ~15;
+        // Gsw = F G X_inf[:, :Ds] = d nuc / d s_w   [Ns][Ds]
+        memset(&a, 0, sizeof a);
+        a.epi = PG_EPI_F32; a.out_f32 = g.Gsw; a.out_f32_stride = static_cast<long long>(N) * D; a.ld_f32 = D; a.n_override = D;
+        PCK(polar_gemm(true, g.FG, Xc, nprob, a, st));
+        // H = X_0 X_inf^T over the student features (the augmentation column left out)
+        memset(&a, 0, sizeof a);
+        a.epi = PG_EPI_SPLIT; a.out_hi = g.Hm.hi; a.out_lo = g.Hm.lo; a.out_stride = g.Hm.batch_stride; a.scale_c = 1.f; a.k_override = d16;
+        PCK(polar_gemm(false, g.X0, Xc, nprob, a, st));
+        // M2 = H G^-1 (I - 1 1^T / Nt),  Theta_raw = G^-T M2
+        memset(&a, 0, sizeof a);
+        a.epi = PG_EPI_SPLIT; a.out_hi = g.M2.hi; a.out_lo = g.M2.lo; a.out_stride = g.M2.batch_stride; a.scale_c = 1.f;
+        PCK(polar_gemm(true, g.Hm, g.GinvC, nprob, a, st));
+        memset(&a, 0, sizeof a);
+        a.epi = PG_EPI_F32; a.out_f32 = g.thraw; a.out_f32_stride = static_cast<long long>(M) * M; a.ld_f32 = M;
+        PCK(polar_gemm(true, g.GinvT, g.M2, nprob, a, st));
+        vt_theta_kernel<<<dim3((M * M + 255) / 256 < 8 ? (M * M + 255) / 256 : 8, nprob), 256, 0, st>>>(g);
+        PCK(cudaGetLastError());
+    }
+    {
+        TimingScope ts(kSlotPolarFinish, st, 1);
         polar_finish_kernel<<<nprob, 256, (2 * N + 64) * sizeof(float), st>>>(g);
         PCK(cudaGetLastError());
-        count += 1;
     }
-    if (launches) *launches = count;
     return cudaSuccess;
 }
 

@@ -102,14 +102,9 @@ polar_fused_abm_kernel(const __grid_constant__ PolarFusedMaps maps, const PolarF
         if (lane == 0) {
             const uint32_t tx = stage_bytes;
             int it = 0, item = 0;
-            if (args.stagger > 0 && (blockIdx.x & 1)) {
-                const long long t0 = clock64();
-                while (clock64() - t0 < args.stagger) __nanosleep(200);
-            }
             for (int w = blockIdx.x; w < args.n_problems; w += gridDim.x, ++item) {
                 const int z = args.reverse ? args.n_problems - 1 - w : w;
                 if (item > 0) mbar_wait(p2done_bar, (item - 1) & 1);       // the operand copy of the previous problem is dead
-                if (args.dbg_clock && blockIdx.x == 0 && item < 16) args.dbg_clock[item * 8 + 0] = clock64();
                 for (int kb = 0; kb < n_kb; ++kb, ++it) {
                     const int s = it % PF_STAGES;
                     const uint32_t ph = (it / PF_STAGES) & 1;
@@ -131,8 +126,6 @@ polar_fused_abm_kernel(const __grid_constant__ PolarFusedMaps maps, const PolarF
         int it = 0, item = 0;
         for (int w = blockIdx.x; w < args.n_problems; w += gridDim.x, ++item) {
             const uint32_t ph_item = item & 1;
-            const bool dbg_m = args.dbg_clock && blockIdx.x == 0 && item < 16 && lane == 0;
-            if (dbg_m) args.dbg_clock[item * 8 + 2] = clock64();
             for (int kb = 0; kb < n_kb; ++kb, ++it) {             // phase 1: A = T W^T
                 const int s = it % PF_STAGES;
                 const uint32_t ph = (it / PF_STAGES) & 1;
@@ -159,10 +152,7 @@ polar_fused_abm_kernel(const __grid_constant__ PolarFusedMaps maps, const PolarF
                     }
                     __syncwarp();
                 }
-                if (lane == 0) {
-                    umma_commit(&empty_bar[s]);
-                    if (kb == n_kb - 1 && dbg_m) args.dbg_clock[item * 8 + 3] = clock64();
-                }
+                if (lane == 0) umma_commit(&empty_bar[s]);
                 __syncwarp();
             }
             if (lane == 0) {                                      // phase 2: acc += (-A~) A~
@@ -171,7 +161,6 @@ polar_fused_abm_kernel(const __grid_constant__ PolarFusedMaps maps, const PolarF
                 // is still reading (generic-proxy writes, fenced by the writers)
                 for (int kb = 0; kb < n_kb2; ++kb) mbar_wait(&copy_bar[kb], ph_item);
                 tc_fence_after();
-                if (dbg_m) args.dbg_clock[item * 8 + 4] = clock64();
                 // row tile by row tile (every operand is resident): tile 0 is stored while tile 1 is still being multiplied
                 for (int mt = 0; mt < args.n_mt; ++mt) {
                     for (int kb = 0; kb < n_kb2; ++kb) {
@@ -189,7 +178,6 @@ polar_fused_abm_kernel(const __grid_constant__ PolarFusedMaps maps, const PolarF
                     umma_commit(&acc2_bar[mt]);
                 }
                 umma_commit(p2done_bar);
-                if (dbg_m) args.dbg_clock[item * 8 + 5] = clock64();
             }
             __syncwarp();
         }
@@ -276,8 +264,6 @@ polar_fused_abm_kernel(const __grid_constant__ PolarFusedMaps maps, const PolarF
             // ---- store: Bm = ca I + (cb r) acc
             mbar_wait(&acc2_bar[mt], ph_item);
             tc_fence_after();
-            const bool dbg_e = args.dbg_clock && blockIdx.x == 0 && item < 16 && e == 0 && lane == 0;
-            if (dbg_e) args.dbg_clock[item * 8 + 6] = clock64();
             const float sc = args.cb * r;
             const int n_ch = (args.bn + 31) / 32;
             for (int ch = 0; ch < n_ch; ++ch) {
@@ -322,8 +308,6 @@ polar_fused_abm_kernel(const __grid_constant__ PolarFusedMaps maps, const PolarF
             __syncwarp();
             tc_fence_before();
             __syncwarp();
-            if (dbg_e) args.dbg_clock[item * 8 + 7] = clock64();
-            if (args.dbg_clock && blockIdx.x == 0 && item < 16 && e == 4 && lane == 0) args.dbg_clock[item * 8 + 1] = clock64();   // tile 1 stored
             if (lane == 0) mbar_arrive(&tmem_empty_bar[mt]);
         }
         if (lane == 0) tma_store_wait_all();

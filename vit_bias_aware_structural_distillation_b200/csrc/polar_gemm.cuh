@@ -64,7 +64,6 @@ struct PolarGemmArgs {
     // auxiliary split matrix laid out like the output, added in the epilogue: out += aux_c * r^aux_p * aux (TMA-loaded)
     int aux_mode; float aux_c, aux_p;
     int a_alias_b;                   // A == B (K-major, same matrix): the A tile is read out of the B tile, no A loads
-    long long* dbg_clock;            // development aid: CTA 0 records clock64() per phase of its first items ([item][8])
     int reverse, n_batches;          // reverse: walk the problems last-to-first (what the previous launch wrote last is still in L2)
     float* trace;                    // if non-null: trace[z][(mt n_nt + nt) 4 + warp] = this warp's share of sum(diag(acc)) (stored, not
                                      // added: the consumer sums the slots in order, so the norm is bitwise repeatable)
@@ -214,8 +213,6 @@ polar_gemm_kernel(const __grid_constant__ typename PgMapsOf<A_TABLE>::type maps,
                 const int mt = itm.mt, z = itm.z;
                 const int a_rows = pg_a_rows(args, mt);
                 const uint32_t tx = (args.a_alias_b ? 0 : a_bufs * a_rows * 128) + 2 * b_bytes;
-                const int item_p = (w - blockIdx.x) / gridDim.x;
-                if (args.dbg_clock && blockIdx.x == 0 && item_p < 16) args.dbg_clock[item_p * 8 + 0] = clock64();
                 for (int kb = 0; kb < n_kb; ++kb, ++it) {
                     const int s = it % args.stages;
                     const uint32_t ph = (it / args.stages) & 1;
@@ -244,7 +241,6 @@ polar_gemm_kernel(const __grid_constant__ typename PgMapsOf<A_TABLE>::type maps,
                         }
                     }
                 }
-                if (args.dbg_clock && blockIdx.x == 0 && item_p < 16) args.dbg_clock[item_p * 8 + 1] = clock64();
             }
         }
     } else if (warp == 1) {
@@ -255,10 +251,8 @@ polar_gemm_kernel(const __grid_constant__ typename PgMapsOf<A_TABLE>::type maps,
             const int acc = item & 1;
             const uint32_t acc_ph = (item >> 1) & 1;
             const int mt_mma = pg_item(args, w).mt;
-            if (args.dbg_clock && blockIdx.x == 0 && item < 16 && lane == 0) args.dbg_clock[item * 8 + 2] = clock64();
             mbar_wait(&tmem_empty_bar[acc], acc_ph ^ 1);           // epilogue has drained this accumulator
             tc_fence_after();
-            if (args.dbg_clock && blockIdx.x == 0 && item < 16 && lane == 0) args.dbg_clock[item * 8 + 3] = clock64();
             const uint32_t d_tmem = tmem_base + acc * args.bn_mma;
             for (int kb = 0; kb < n_kb; ++kb, ++it) {
                 const int s = it % args.stages;
@@ -284,7 +278,6 @@ polar_gemm_kernel(const __grid_constant__ typename PgMapsOf<A_TABLE>::type maps,
                     }
                     umma_commit(&empty_bar[s]);
                     if (kb == n_kb - 1) umma_commit(&tmem_full_bar[acc]);
-                    if (args.dbg_clock && blockIdx.x == 0 && item < 16 && kb == n_kb - 1) args.dbg_clock[item * 8 + 4] = clock64();
                 }
                 __syncwarp();
             }
@@ -322,10 +315,8 @@ polar_gemm_kernel(const __grid_constant__ typename PgMapsOf<A_TABLE>::type maps,
                 tma_load_3d(sg_tile, &maps.o[2], &aux_bar[warp - 2], c0, mt * 128 + q * 32, z);
                 tma_load_3d(sg_tile + 4096, &maps.o[2], &aux_bar[warp - 2], c0 + 32, mt * 128 + q * 32, z);
             }
-            if (args.dbg_clock && blockIdx.x == 0 && item < 16 && warp == 2 && lane == 0) args.dbg_clock[item * 8 + 5] = clock64();
             mbar_wait(&tmem_full_bar[acc], acc_ph);
             tc_fence_after();
-            if (args.dbg_clock && blockIdx.x == 0 && item < 16 && warp == 2 && lane == 0) args.dbg_clock[item * 8 + 6] = clock64();
             const uint32_t t_addr = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + acc * args.bn_mma;
             const int row = mt * 128 + q * 32 + lane;
             const bool row_ok = row < args.m_rows;
@@ -376,8 +367,6 @@ polar_gemm_kernel(const __grid_constant__ typename PgMapsOf<A_TABLE>::type maps,
                     const uint8_t* aux_hi_s = aux_base + cbk * 8192;
                     const uint8_t* aux_lo_s = aux_hi_s + 4096;
                     // whole 64-column block in one tcgen05.ld (the last block of a 208-wide tile has 16 columns)
-                    const bool dbg_here = args.dbg_clock && blockIdx.x == 0 && item == 5 && cbk == 1 && warp == 2 && lane == 0;
-                    if (dbg_here) args.dbg_clock[120] = clock64();
                     float vb[64];
                     const int cols_here = min(64, args.bn_mma - cbk * 64);
                     float4 sg_g[kSgrad ? 16 : 1];
@@ -405,7 +394,6 @@ polar_gemm_kernel(const __grid_constant__ typename PgMapsOf<A_TABLE>::type maps,
                             if (jc * 16 < cols_here) tmem_ld16(t_addr + cbk * 64 + jc * 16, vb + jc * 16);
                         }
                     }
-                    if (dbg_here) args.dbg_clock[121] = clock64();
 #pragma unroll
                     for (int jc = 0; jc < 4; ++jc) {
                         const int c = c0 + cbk * 64 + jc * 16;                  // global column of v[0]
@@ -468,10 +456,8 @@ polar_gemm_kernel(const __grid_constant__ typename PgMapsOf<A_TABLE>::type maps,
                             pg_stage_zero16(stg_hi_s, stg_lo_s, lane, jc * 2);      // padding columns of the last block
                         }
                     }
-                    if (dbg_here) args.dbg_clock[122] = clock64();
                     fence_proxy_async_smem();
                     __syncwarp();                                               // staging complete; aux tile fully consumed
-                    if (dbg_here) args.dbg_clock[123] = clock64();
                     if (lane == 0 && warp_rows_ok) {
                         if constexpr (kF32Staged) {                             // two 32 x 32 fp32 boxes; columns past n_cols / rows past m_rows are clipped
                             tma_store_3d(&maps.o[0], stg_hi, c0 + cbk * 64, mt * 128 + q * 32, z);
@@ -488,9 +474,7 @@ polar_gemm_kernel(const __grid_constant__ typename PgMapsOf<A_TABLE>::type maps,
                             tma_store_4d(&maps.o[1], stg_lo, 0, mt * 128 + q * 32, cb0 + cbk, z);
                         }
                         tma_store_commit();
-                        if (dbg_here) args.dbg_clock[124] = clock64();
                         tma_store_wait_read();
-                        if (dbg_here) args.dbg_clock[125] = clock64();
                     }
                     __syncwarp();
                 }
@@ -515,7 +499,6 @@ polar_gemm_kernel(const __grid_constant__ typename PgMapsOf<A_TABLE>::type maps,
             }
             tc_fence_before();
             __syncwarp();
-            if (args.dbg_clock && blockIdx.x == 0 && item < 16 && warp == 2 && lane == 0) args.dbg_clock[item * 8 + 7] = clock64();
             if (lane == 0) mbar_arrive(&tmem_empty_bar[acc]);
             if (args.trace) {
 #pragma unroll

@@ -8,7 +8,6 @@
 #include "spectral.h"
 
 #include <math_constants.h>
-#include <cstdlib>
 #include <cstring>
 #include <mutex>
 #include <vector>
@@ -17,22 +16,6 @@
 #include "jacobi.cuh"
 
 namespace basd {
-
-// development aid (tools/gpu_debug_eig.py): phase clocks of the first pooled_eig cluster [0..7] and of angles CTA (0,0) [8..23]
-__device__ long long g_spectral_clk[32];
-__device__ int g_spectral_dbg_on;                      // written once by the host when BASD_SPECTRAL_DBG is set; otherwise no launch touches g_spectral_clk
-static void spectral_dbg_init() {
-    static const bool once = [] {
-        const char* e = getenv("BASD_SPECTRAL_DBG");      // value = 1 + the teacher layer whose angles CTA is recorded
-        const int on = e ? (atoi(e) > 0 ? atoi(e) : 1) : 0;
-        if (on) cudaMemcpyToSymbol(g_spectral_dbg_on, &on, sizeof(int));
-        return true;
-    }();
-    (void)once;
-}
-int spectral_debug_clocks(long long* host_out) {
-    return cudaMemcpyFromSymbol(host_out, g_spectral_clk, sizeof(long long) * 32) == cudaSuccess ? 0 : 1;
-}
 
 constexpr float kJacobiTol = 3.0e-7f;
 constexpr int kJacobiMaxSweeps = 40;
@@ -182,7 +165,6 @@ pooled_eig_kernel(const float* __restrict__ stats, int n, int Lt, int P, float M
     __shared__ __align__(8) uint64_t s_bars[2];
     __shared__ int s_bad;
 
-    const long long t_begin = clock64();
     const int crank = LARGE ? 0 : static_cast<int>(cooperative_groups::this_cluster().block_rank());
     const int p = LARGE ? blockIdx.x : blockIdx.x / static_cast<int>(cooperative_groups::this_cluster().num_blocks());
     const bool mp_mode = mode == kEigMpOnly;
@@ -226,7 +208,6 @@ pooled_eig_kernel(const float* __restrict__ stats, int n, int Lt, int P, float M
     }
     __syncthreads();
     }   // crank == 0
-    const long long t_pre = clock64();
     int nsweeps = 0;
     if constexpr (LARGE) {
         if (phase == 0) {
@@ -243,7 +224,6 @@ pooled_eig_kernel(const float* __restrict__ stats, int n, int Lt, int P, float M
         if (crank != 0) return;                 // (the Jacobi routine ends with a cluster barrier: nobody touches this CTA again)
         if (!cluster_ok) nsweeps = run_jacobi(A, ld, n);
     }
-    const long long t_jac = clock64();
     column_norms(A, ld, n, n, vals);        // sigma_i (Cholesky route) or lambda_i (fallback)
     __syncthreads();
     if (use_chol)
@@ -313,7 +293,6 @@ pooled_eig_kernel(const float* __restrict__ stats, int n, int Lt, int P, float M
     // eigenvector e = column order[e] of A, normalised; one warp per eigenvector, lanes over components (conflict-free
     // shared reads; the [eig][comp] store is coalesced, the [comp][eig] one is a 4-byte scatter that L2 merges)
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nwarps = blockDim.x >> 5;
-    if (threadIdx.x == 0 && p == 0 && g_spectral_dbg_on) { g_spectral_clk[0] = t_pre - t_begin; g_spectral_clk[1] = t_jac - t_pre; g_spectral_clk[2] = clock64() - t_jac; g_spectral_clk[3] = nsweeps; }
     for (int e = warp; e < n; e += nwarps) {
         const float* col = A + static_cast<size_t>(order[e]) * ld;
         const float s = csum[e];
@@ -393,14 +372,11 @@ angles_kernel(int n, int Lt, int P, const int* __restrict__ ranks, const float* 
     float* Fg = WQg + n * n;                  // [a][e]
     float* T1g = Fg + n * n;                  // H [a][c]
 
-    const bool dbg = static_cast<int>(blockIdx.x) == g_spectral_dbg_on - 1 && blockIdx.y == 0 && threadIdx.x == 0 && g_spectral_dbg_on;
-    if (dbg) g_spectral_clk[31] = k;
     if (k == 0) {                              // reference: 0/0 -> NaN (layer_selector.py:105)
         if (threadIdx.x == 0) d2_out[i * Lt + j] = CUDART_NAN_F;
         for (int t = threadIdx.x; t < n * n; t += blockDim.x) gam[t] = 0.f;
         return;
     }
-    if (dbg) g_spectral_clk[8 + 0] = clock64();
     // (a) Ur[b][c] = sum_r Ut[b][r] P_s[r][c]
     const bool vec_ok = (n & 3) == 0;                  // 128-bit operand loads (cta_gemm_mk); every D_s the library accepts is a multiple of 8
     if (vec_ok) {
@@ -414,7 +390,6 @@ angles_kernel(int n, int Lt, int P, const int* __restrict__ ranks, const float* 
     __syncthreads();
     for (int t = threadIdx.x; t < ld * k; t += blockDim.x) J[t] = 0.f;
     __syncthreads();
-    if (dbg) g_spectral_clk[8 + 1] = clock64();
     // (b) W[e][b] = sum_c Vs[e][c] Ur[b][c];   its top k x k block is A = V_s[:, :k]^T (P_s^T U_t)
     //     J = A^T goes straight to shared memory: column a of J = row a of A
     if (vec_ok) {
@@ -426,25 +401,21 @@ angles_kernel(int n, int Lt, int P, const int* __restrict__ ranks, const float* 
                  [&](int e, int b, float v) { Wg[b * n + e] = v; if (e < k) J[e * ld + b] = v; });
     }
     __syncthreads();
-    if (dbg) g_spectral_clk[8 + 2] = clock64();
-    if (dbg) g_spectral_clk[8 + 3] = clock64();
     // (c) one-sided Jacobi on A^T:  A^T R = Y Sigma  =>  A^T A = Y Sigma^2 Y^T.  The rotated columns are sigma_m y_m: their
     //     norms are the cosines themselves (no squaring through A^T A) and their directions the right singular vectors.
     // odd-even ordering with register-resident columns (a "cluster" of this one CTA): half the shared-memory round trips
     // and barriers of the round-robin version per rotation; k x k with k ~ 15-40 is a pure latency chain
-    int nsw = 0;
     if (!j_in_smem) {
         __threadfence_block();
-        nsw = run_jacobi_global(J, ld, k);
+        run_jacobi_global(J, ld, k);
     } else {
+        int nsw;
         if (!run_jacobi_oddeven_cluster(J, ld, k, inbox, s_bars, s_flags, &nsw)) run_jacobi(J, ld, k);
     }
-    if (dbg) g_spectral_clk[30] = nsw;
     column_norms(J, ld, k, k, vals);          // vals = sigma
     __syncthreads();
     rank_descending(vals, k, order);
     __syncthreads();
-    if (dbg) g_spectral_clk[8 + 4] = clock64();
     // (d) distances and d(d2)/dsigma
     float swsum = 0.f, acc = 0.f;
     for (int r = threadIdx.x; r < k; r += blockDim.x) swsum += sqrtf(fmaxf(lam_t[r], 0.f));
@@ -466,7 +437,6 @@ angles_kernel(int n, int Lt, int P, const int* __restrict__ ranks, const float* 
     acc = cta_sum(acc, red);
     if (threadIdx.x == 0) d2_out[i * Lt + j] = acc / swsum;
     __syncthreads();
-    if (dbg) g_spectral_clk[8 + 5] = clock64();
     // Q[b][b'] = sum_m J[b][m] coef_m J[b'][m]     (rows kq = k rounded up to 4 apart: 16-byte aligned for the 128-bit loads below)
     const int kq = (k + 3) & ~3;
     cta_gemm(k, k, k,
@@ -474,7 +444,6 @@ angles_kernel(int n, int Lt, int P, const int* __restrict__ ranks, const float* 
              [&](int m, int b2) { return J[m * ld + b2]; },
              [&](int b, int b2, float v) { Qg[b2 * kq + b] = v; });
     __syncthreads();
-    if (dbg) g_spectral_clk[8 + 6] = clock64();
     // (e) WQ[e][b'] = sum_b W[e][b] Q[b][b']
     if (vec_ok) {
         cta_gemm_mk(n, k, k, Wg, n, Qg, kq, [&](int e, int b2, float v) { WQg[b2 * n + e] = v; });
@@ -485,7 +454,6 @@ angles_kernel(int n, int Lt, int P, const int* __restrict__ ranks, const float* 
                  [&](int e, int b2, float v) { WQg[b2 * n + e] = v; });
     }
     __syncthreads();
-    if (dbg) g_spectral_clk[8 + 7] = clock64();
     //     F[e][a] = (sum_b' WQ[e][b'] A[a][b']) / (lam_a - lam_e)   for e >= k, a < k
     const int nc = n - k;
     cta_gemm(nc, k, k,
@@ -493,7 +461,6 @@ angles_kernel(int n, int Lt, int P, const int* __restrict__ ranks, const float* 
              [&](int b2, int a) { return Wg[b2 * n + a]; },
              [&](int e, int a, float v) { Fg[a * n + e] = v / (lam_s[a] - lam_s[k + e]); });      // (row a of F from column 0: aligned)
     __syncthreads();
-    if (dbg) g_spectral_clk[8 + 8] = clock64();
     // (f) Gamma = V_hi^T F V_lo  (V_hi = eigenvectors e >= k, V_lo = a < k), associated as (V_hi^T F) V_lo: n k (n + nc)
     //     multiply-adds instead of the n n nc of V_hi^T (F V_lo), k << nc.
     //     H[c][a] = sum_{e>=k} Vs[e][c] F[e][a]
@@ -506,7 +473,6 @@ angles_kernel(int n, int Lt, int P, const int* __restrict__ ranks, const float* 
                  [&](int c, int a, float v) { T1g[a * n + c] = v; });
     }
     __syncthreads();
-    if (dbg) g_spectral_clk[8 + 9] = clock64();
     //     Gamma_sym[c][c'] = sum_a H[c][a] Vs[a][c'] + Vs[a][c] H[c'][a]   (one product of inner size 2k; symmetric, so the
     //     store may run along c)
     if ((n & 3) == 0) {
@@ -535,8 +501,6 @@ angles_kernel(int n, int Lt, int P, const int* __restrict__ ranks, const float* 
                  [&](int a, int c2) { return a < k ? Vs_km[a * n + c2] : T1g[(a - k) * n + c2]; },
                  [&](int c, int c2, float v) { gam[c2 * n + c] = v; });
     }
-    if (dbg) g_spectral_clk[8 + 10] = clock64();
-    if (dbg) g_spectral_clk[8 + 11] = clock64();
 }
 
 // w = softmax(-d2 / softplus(log_temperature))   one warp per extraction point
@@ -646,14 +610,8 @@ size_t pooled_eig_scratch_floats(int n, int problems) { return spectral_large(n)
 // (24 problems on 6-CTA clusters, then the last 4 on 8-CTA clusters) measured 10.2 ms (r3c): in ONE launch the remaining clusters
 // start as soon as any problem converges, the split makes them wait for the slowest of the first 24.
 static int pooled_pick_cluster(const void* kern, int n, int problems, size_t smem_fixed, size_t smem_per_group_floats) {
-    static const int forced = [] {            // BASD_EIG_CLUSTER: development knob (1..8 CTAs per problem), read once
-        const char* env = getenv("BASD_EIG_CLUSTER");
-        const int c = env ? atoi(env) : 0;
-        return (c < 1 || c > 8) ? 0 : c;
-    }();
     const int groups = (n + 1) / 2, per_cta = kPooledThreads / JAC_GROUP;
     const int c_min = (groups + per_cta - 1) / per_cta;
-    if (forced) return forced < c_min ? c_min : forced;
     struct Key { int dev, n, problems, cluster; const void* kern; };
     static std::mutex mu;
     static std::vector<Key> cache;
@@ -684,7 +642,6 @@ static int pooled_pick_cluster(const void* kern, int n, int problems, size_t sme
 
 cudaError_t launch_pooled_eig(const float* stats, int n, int Lt, int P, float Mt, float Ms, int* ranks, float* evals,
                               float* evecs_km, float* evecs_cm, int* sweeps, float* scratch, cudaStream_t st, int mode) {
-    spectral_dbg_init();
     const bool large = spectral_large(n);
     const size_t smem = pooled_smem(n, large);
     const int problems = mode == kEigMpOnly ? Lt : Lt + P;

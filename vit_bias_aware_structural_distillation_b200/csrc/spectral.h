@@ -155,8 +155,6 @@ struct PolarFusedArgs {
     float* fro2;                     // [problem][fro_slots]: slot 0 written here
     int fro_slots;
     float* resid;                    // last step only: [problem][fro_slots] per-warp partial sums of ||A - I||_F^2 (else null)
-    long long* dbg_clock;            // development aid: CTA 0 records clock64() per phase of its first problems ([problem][8])
-    int stagger;                     // development aid (BASD_POLAR_FUSED_STAGGER): odd CTAs start their first loads this many cycles late
 };
 // Bm = ca I + cb (rA) + cc (rA)^2 with A = T W^T kept on chip (polar_fused.cuh); needs polar_fused_supported(D_s, N_s)
 bool polar_fused_supported(int n, int k);
@@ -202,8 +200,8 @@ struct PolarArgs {
     float* loss_b;                        // [P*B]
     float* dbg;                           // [P*B][5]
 };
-cudaError_t launch_polar_procrustes(const PolarArgs& args, cudaStream_t st, int* launches);
-cudaError_t launch_polar_procrustes_vt(const PolarArgs& args, cudaStream_t st, int* launches);
+cudaError_t launch_polar_procrustes(const PolarArgs& args, cudaStream_t st);
+cudaError_t launch_polar_procrustes_vt(const PolarArgs& args, cudaStream_t st);
 constexpr int kVtMaxTokens = 224;         // teacher tokens of the token-space form (Cholesky factor held in shared memory)
 int polar_fro_slots(int core);            // partial-trace slots per problem for a core (D_s or N_t) of this size
 constexpr int kPolarStepsDefault = 10, kPolarStepsMin = 7, kPolarStepsMax = 16;   // (fewer than the default: caller override only, rows of the schedule skipped from the front)

@@ -1,12 +1,11 @@
 // Warp-specialised tcgen05 GEMM for sm_100a: TMA (SWIZZLE_128B) -> shared memory ring -> tcgen05.mma
 // (bf16 x bf16 -> fp32 in TMEM) -> tcgen05.ld epilogue.  One CTA = MT x (128 x BN) output tiles.
 //
-// Every dense contraction of the BASD loss path is an instance (see gemm_ops.cu):
-//   project      Z = X P_t^T                 (replaces layer_selector.py:72,135)      A,B K-major
+// Instances on the BASD loss path (see gemm_ops.cu):
 //   gram         G += Z_chunk^T Z_chunk      (replaces layer_selector.py:13,36,92)    A,B MN-major, split-K
-//   token_gram   K = T T^T per sample        (relational.py:47 moved to token space)  A,B K-major, B aliases A
-//   (theta_apply D = Theta T per sample runs on the persistent polar_gemm kernel: gemm_ops.cu)
-//   student_grad dS = S Gamma + ...          (SURVEY.md B.5)                          A,B K-major
+//   token_gram   K = T T^T per sample        (relational.py:47 moved to token space)  A,B K-major, B aliases A; N_s < 16 only
+//   student_grad dS = S Gamma + ...          (SURVEY.md B.5)                          A,B K-major; views, fp32 or split students
+//   (project, the other token Grams, theta_apply and the dense bf16 student gradient run on the persistent polar_gemm kernel)
 // "Split-bf16" terms (hi/lo operand pairs) accumulate into the same TMEM tile to recover fp32-class
 // accuracy from bf16 tensor-core passes.
 #pragma once
@@ -46,7 +45,7 @@ struct GemmArgs {
     float beta;
     // Row-gapped A operand (K-major, rows = M): a [B][N+1][D] buffer read through its CLS-stripped view [:,1:,:] is a dense
     // 2-D matrix whose rows r with r % gap_period >= gap_valid belong to no sample (trainer.py:29, teacher.py:157 hand such
-    // views over).  gap_period == 0: no gaps.  Epilogues zero (project) or skip (student_grad) those rows.
+    // views over).  gap_period == 0: no gaps.  The student_grad epilogue skips those rows.
     int gap_period, gap_valid;
     // MN-major operands whose K dimension runs over the rows of a [B][N][D] tensor with an arbitrary batch stride: the tensor
     // map is 3-D (D, N, B) and k-block kb covers rows (kb % kb_per_batch) * 64.. of sample kb / kb_per_batch; rows past N are
@@ -252,46 +251,6 @@ umma_gemm_kernel(const __grid_constant__ GemmMaps maps, const GemmArgs args) {
 // ---------------------------------------------------------------------------------------------------
 // Epilogues.  operator()(row, col0, v[16]) handles 16 consecutive columns of one output row.
 // ---------------------------------------------------------------------------------------------------
-struct EpiStoreSplit {                    // out = hi, aux0 = lo:  hi = bf16(acc), lo = bf16(acc - hi)   (fp32-class storage)
-    __nv_bfloat16* hi; __nv_bfloat16* lo; int ld, rows, cols, gap_period, gap_valid;
-    __device__ EpiStoreSplit(const GemmArgs& a, int batch, int) {
-        hi = reinterpret_cast<__nv_bfloat16*>(a.out) + batch * a.out_batch_stride;
-        lo = reinterpret_cast<__nv_bfloat16*>(const_cast<void*>(a.aux0)) + batch * a.out_batch_stride;
-        ld = a.ld_out; rows = a.rows_valid; cols = a.cols_valid; gap_period = a.gap_period; gap_valid = a.gap_valid;
-    }
-    __device__ void operator()(int row, int col0, const float* vin) const {
-        if (row >= rows || col0 >= cols) return;
-        const long long off = static_cast<long long>(row) * ld + col0;
-        float vz[16];
-        const float* v = vin;
-        if (gap_period && row % gap_period >= gap_valid) {          // a row between two samples (another sample's CLS token): zeros,
-#pragma unroll
-            for (int i = 0; i < 16; ++i) vz[i] = 0.f;               // so the Gram and the column sums over these rows are unaffected
-            v = vz;
-        }
-        if (col0 + 16 <= cols) {
-            uint32_t hw[8], lw[8];
-#pragma unroll
-            for (int i = 0; i < 8; ++i) {
-                const __nv_bfloat16 h0 = __float2bfloat16(v[2 * i]), h1 = __float2bfloat16(v[2 * i + 1]);
-                __nv_bfloat162 hv; hv.x = h0; hv.y = h1;
-                hw[i] = *reinterpret_cast<uint32_t*>(&hv);
-                lw[i] = pack_bf16x2(v[2 * i] - __bfloat162float(h0), v[2 * i + 1] - __bfloat162float(h1));
-            }
-            reinterpret_cast<uint4*>(hi + off)[0] = make_uint4(hw[0], hw[1], hw[2], hw[3]);
-            reinterpret_cast<uint4*>(hi + off)[1] = make_uint4(hw[4], hw[5], hw[6], hw[7]);
-            reinterpret_cast<uint4*>(lo + off)[0] = make_uint4(lw[0], lw[1], lw[2], lw[3]);
-            reinterpret_cast<uint4*>(lo + off)[1] = make_uint4(lw[4], lw[5], lw[6], lw[7]);
-        } else {
-            for (int i = 0; i < 16 && col0 + i < cols; ++i) {
-                const __nv_bfloat16 h = __float2bfloat16(v[i]);
-                hi[off + i] = h;
-                lo[off + i] = __float2bfloat16(v[i] - __bfloat162float(h));
-            }
-        }
-    }
-};
-
 struct EpiStoreF32 {                      // out[batch][row][col] = alpha * acc
     float* out; int ld, rows, cols; float alpha;
     __device__ EpiStoreF32(const GemmArgs& a, int batch, int) {
